@@ -377,7 +377,7 @@ int sbgm_upsample2x_backward(const void* dy, size_t dy_plane, void* dx, size_t d
                              void* stream);
 /* attention core backward: dqkv [b*s][3c] from qkv, the forward's output `out` [b*s][c] (NULL: not available) and dout
  * [b*s][c].  bf16 with S % 16 == 0 and head dim 32 / 64 / 128 (and `out` given): ONE warp-level tensor-core launch, a CTA
- * per (image, head), nothing but dqkv written (attention_bwd_mma.cu; SBGM_B200_ATTN_BWD_MMA=0 disables).  Otherwise: fp32
+ * per (image, head), nothing but dqkv written (attention_bwd_mma.cu).  Otherwise: fp32
  * batched CUDA-core GEMMs from `scratch` (..._scratch_floats floats; unused by the tensor-core path). */
 size_t sbgm_attention_backward_scratch_floats(int b, int s, int c, int heads);
 int sbgm_attention_backward(const void* qkv, size_t qkv_plane, const void* out, size_t out_plane, const void* dout, size_t dout_plane,
@@ -411,16 +411,6 @@ int sbgm_conv2d_wgrad_simt(const void* x, size_t x_plane, const void* dy, size_t
 size_t sbgm_conv2d_wgrad_tc_workspace_floats(int fmt, int n, int h, int w, int cin, int cout, int kh, int kw, int stride, int pad);
 int sbgm_conv2d_wgrad_tc(const void* x, size_t x_plane, const void* dy, size_t dy_plane, float* dweight_oihw, int fmt,
                          int n, int h, int w, int cin, int cout, int kh, int kw, int stride, int pad, float* workspace, void* stream);
-/* Deferred form: sbgm_conv2d_wgrad_tc with dweight_oihw = NULL leaves its sbgm_conv2d_wgrad_tc_splits(...) partial slabs
- * [splits][cout][kh*kw*cin] in `workspace`; sbgm_wgrad_reduce_batch then sums the slabs of MANY layers in one launch into their
- * OIHW gradients (46 per-layer reduce launches of a training step become one per decoder block / encoder stage). */
-int sbgm_conv2d_wgrad_tc_splits(int fmt, int n, int h, int w, int cin, int cout, int kh, int kw, int stride, int pad);
-typedef struct {
-  const float* workspace;
-  float* dweight_oihw;
-  int splits, cout, taps, cin;
-} sbgm_wgrad_reduce_job;
-int sbgm_wgrad_reduce_batch(const sbgm_wgrad_reduce_job* jobs_host, int njobs, void* stream);
 /* sum workspace[splits][cout][taps*cin] over the splits in a fixed order into OIHW */
 int sbgm_wgrad_reduce(const float* workspace, int splits, int cout, int taps, int cin, float* dweight_oihw, void* stream);
 /* Encoder.conv1 (8x8 s2 p3 over NCHW fp32 x || planes, score_unet.py:310): weight gradient from df [n,h/2,w/2,64] */

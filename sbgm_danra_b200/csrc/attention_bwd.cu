@@ -176,11 +176,9 @@ int sbgm_attention_backward(const void* qkv, size_t qkv_plane, const void* out, 
   SBGM_REQUIRE(heads >= 1 && c % heads == 0 && (c / heads) % 8 == 0, "attention_backward: bad c=%d heads=%d", c, heads);
   cudaStream_t st = as_stream(stream);
   (void)out_plane;
-  static const bool mma_on = [] { const char* e = getenv("SBGM_B200_ATTN_BWD_MMA"); return !(e != nullptr && e[0] == '0'); }();
-  if (mma_on) {      // bf16, S % 16 == 0, head dim 32 / 64 / 128: one tensor-core launch
-    const int rc = attention_bwd_mma_dispatch(qkv, out, dout, dqkv, fmt, b, s, c, heads, st);
-    if (rc >= 0) return rc;
-  }
+  // bf16, S % 16 == 0, head dim 32 / 64 / 128: one tensor-core launch
+  const int mma_rc = attention_bwd_mma_dispatch(qkv, out, dout, dqkv, fmt, b, s, c, heads, st);
+  if (mma_rc >= 0) return mma_rc;
   const int d = c / heads, bh = b * heads;
   const size_t tok = static_cast<size_t>(b) * s * c, mat = static_cast<size_t>(bh) * s * s;
   float* q = scratch;

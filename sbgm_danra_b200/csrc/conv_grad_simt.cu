@@ -141,49 +141,6 @@ __global__ void wgrad_reduce_kernel(const float* __restrict__ ws, int splits, in
   }
 }
 
-// The same reduction for MANY layers in one launch (a decoder block's or an encoder stage's worth of weight gradients): per
-// layer the reduce is a 3-7 us latency-bound kernel behind a ~1.9 us kernel boundary, 46 of them per training step; batched,
-// the GPU is filled once and the sum of the partial slabs streams at HBM rate.  Jobs travel as a kernel parameter.
-constexpr int kReduceBatch = 64;
-struct ReduceJobDev {
-  const float* ws;
-  float* out;
-  unsigned long long item_end;     // running total of output elements up to and including this job
-  uint32_t total;                  // cout * taps * cin
-  uint16_t splits, taps;
-  uint32_t cin;
-};
-struct ReduceBatch {
-  int njobs;
-  ReduceJobDev jobs[kReduceBatch];
-};
-__global__ void __launch_bounds__(256) wgrad_reduce_batch_kernel(const __grid_constant__ ReduceBatch b) {
-  pdl_grid_sync();
-  // an item = four consecutive input channels of one (co, tap): one 16-byte load per slab, four slabs in flight per thread
-  const unsigned long long items = b.jobs[b.njobs - 1].item_end;
-  for (unsigned long long v = blockIdx.x * 256ull + threadIdx.x; v < items; v += static_cast<unsigned long long>(gridDim.x) * 256ull) {
-    int lo = 0, hi = b.njobs - 1;
-    while (lo < hi) {
-      const int mid = (lo + hi) >> 1;
-      if (b.jobs[mid].item_end > v) hi = mid; else lo = mid + 1;
-    }
-    const ReduceJobDev& j = b.jobs[lo];
-    const uint32_t i = 4u * static_cast<uint32_t>(v - (lo > 0 ? b.jobs[lo - 1].item_end : 0ull));
-    const uint32_t K = static_cast<uint32_t>(j.taps) * j.cin;
-    const uint32_t ci = i % j.cin, tap = (i / j.cin) % j.taps, co = i / K;
-    float4 acc = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
-    const float4* src = reinterpret_cast<const float4*>(j.ws + i);
-    const size_t slab = j.total >> 2;
-#pragma unroll 4
-    for (int z = 0; z < j.splits; ++z) {
-      const float4 p = __ldg(src + static_cast<size_t>(z) * slab);
-      acc.x += p.x; acc.y += p.y; acc.z += p.z; acc.w += p.w;
-    }
-    float* o = j.out + (static_cast<size_t>(co) * j.cin + ci) * j.taps + tap;
-    o[0] = acc.x; o[j.taps] = acc.y; o[2 * j.taps] = acc.z; o[3 * j.taps] = acc.w;
-  }
-}
-
 // ---- stem wgrad --------------------------------------------------------------------------------------
 // ws[chunk][ci][tap][co] = sum over the chunk's output pixels of df1[p][co] * in[n][ci][2 oy + r - 3][2 ox + s - 3]
 constexpr int kStemChunks = 64;
@@ -577,30 +534,6 @@ int sbgm_wgrad_reduce(const float* workspace, int splits, int cout, int taps, in
   const size_t total = static_cast<size_t>(cout) * taps * cin;
   launch_k((wgrad_reduce_kernel), cgrid_for(total, 256), 256, 0, as_stream(stream), workspace, splits, cout, taps, cin, dweight_oihw);
   return check_launch("wgrad_reduce");
-}
-
-int sbgm_wgrad_reduce_batch(const sbgm_wgrad_reduce_job* jobs_host, int njobs, void* stream) {
-  cudaStream_t st = as_stream(stream);
-  for (int base = 0; base < njobs; base += kReduceBatch) {
-    ReduceBatch b;
-    b.njobs = (njobs - base < kReduceBatch) ? njobs - base : kReduceBatch;
-    unsigned long long items = 0;
-    for (int k = 0; k < b.njobs; ++k) {
-      const sbgm_wgrad_reduce_job& h = jobs_host[base + k];
-      const unsigned long long total = static_cast<unsigned long long>(h.cout) * h.taps * h.cin;
-      SBGM_REQUIRE(h.workspace != nullptr && h.dweight_oihw != nullptr && h.splits >= 1 && h.splits <= 65535 && h.taps >= 1 && h.taps <= 65535 &&
-                       h.cin >= 1 && h.cout >= 1 && total < (1ull << 32),
-                   "wgrad_reduce_batch: bad job %d (splits %d, cout %d, taps %d, cin %d)", base + k, h.splits, h.cout, h.taps, h.cin);
-      SBGM_REQUIRE(h.cin % 4 == 0 && (reinterpret_cast<uintptr_t>(h.workspace) & 15) == 0,
-                   "wgrad_reduce_batch: job %d needs cin %% 4 == 0 and a 16-byte aligned workspace", base + k);
-      items += total / 4;
-      ReduceJobDev& d = b.jobs[k];
-      d.ws = h.workspace; d.out = h.dweight_oihw; d.item_end = items; d.total = static_cast<uint32_t>(total);
-      d.splits = static_cast<uint16_t>(h.splits); d.taps = static_cast<uint16_t>(h.taps); d.cin = static_cast<uint32_t>(h.cin);
-    }
-    launch_k((wgrad_reduce_batch_kernel), cgrid_for(items, 256, 148 * 16), 256, 0, st, b);
-  }
-  return check_launch("wgrad_reduce_batch");
 }
 
 size_t sbgm_stem_wgrad_workspace_floats(int cin) { return static_cast<size_t>(kStemChunks) * cin * 64 * 64; }

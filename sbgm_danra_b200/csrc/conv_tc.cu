@@ -794,22 +794,19 @@ static int conv2d_tc_impl(const void* in, size_t in_plane, const void* weight, s
   p.ep.proj_w = proj_w; p.ep.proj_out = proj_out; p.ep.n_proj = n_proj;
   SBGM_REQUIRE(p.w_tile * stride <= 256 && p.h_tile * stride <= 256, "conv2d_tc: TMA box too large for stride %d", stride);
 
-  // dense output addressing, full epilogue: the tile leaves through shared memory and TMA stores (SBGM_B200_TMA_STORE=0: off)
-  static const bool tma_store_on = [] { const char* e = getenv("SBGM_B200_TMA_STORE"); return !(e != nullptr && e[0] == '0'); }();
-  p.ep.staged = ((tma_store_on || ln_colsum != nullptr) && !scatter && proj_w == nullptr && p.splits == 1 && out != nullptr) ? 1 : 0;
-  // 3x3 / stride 1 / pad 1: one halo slab per 64-channel block (SBGM_B200_SLAB=0: off).  Maps tileable by 16 rows x 8 columns
+  // dense output addressing, full epilogue: the tile leaves through shared memory and TMA stores
+  p.ep.staged = (!scatter && proj_w == nullptr && p.splits == 1 && out != nullptr) ? 1 : 0;
+  // 3x3 / stride 1 / pad 1: one halo slab per 64-channel block.  Maps tileable by 16 rows x 8 columns
   // use 16 x 8 tiles of one image; other maps tileable by 8 x 8 use 8 x 8 tiles of two images with permuted tensor maps
   // (no fused GroupNorm statistics there: a warp's 32 rows span two images).  Split-K slices the 64-channel blocks.
-  static const bool slab_on = [] { const char* e = getenv("SBGM_B200_SLAB"); return !(e != nullptr && e[0] == '0'); }();
-  bool slab = slab_on && (p.ep.staged || (p.splits > 1 && proj_w == nullptr && !scatter)) && kh == 3 && kw == 3 && stride == 1 &&
+  bool slab = (p.ep.staged || (p.splits > 1 && proj_w == nullptr && !scatter)) && kh == 3 && kw == 3 && stride == 1 &&
               p.pad_h == 1 && p.pad_w == 1 && ho == h && wo == w && wo % 8 == 0 && ho % 8 == 0;
   const bool slab_perm = slab && ho % kSlabTileH != 0;
   if (slab_perm && gn_partials != nullptr) slab = false;
   if (slab && p.splits > 1 && (p.splits - 1) * ceil_div(p.cin_blocks, p.splits) >= p.cin_blocks) slab = false;
   // slab mode makes the activation operand cheap to re-read: a two-way split-K 128-wide layer (the 8 x 8 maps) runs instead as
   // twice as many 64-wide tiles over the whole K loop -- same CTA count, no partial tiles, no finalize kernel
-  static const bool nosplit_on = [] { const char* e = getenv("SBGM_B200_SLAB_NOSPLIT"); return !(e != nullptr && e[0] == '0'); }();
-  if (slab && nosplit_on && p.splits == 2 && block_n == 128 && tma_store_on && out != nullptr) {
+  if (slab && p.splits == 2 && block_n == 128 && out != nullptr) {
     block_n = 64;
     p.splits = 1;
     p.ep.staged = 1;
@@ -826,28 +823,24 @@ static int conv2d_tc_impl(const void* in, size_t in_plane, const void* weight, s
   // Two pixel tiles per CTA (MT = 2) where the grid stays full (>= 1.7 waves of one-tile CTAs): the weight boxes -- most of a
   // K-heavy layer's operand bytes -- are fetched once for both.  Measured per layer (profiles/r02_conv_tc_family_table_*.txt):
   // conv2 110 -> 66 us, 128->128 at 32 x 32 47 -> 42 us; trading a 128-wide one-wave grid for 64-wide two-tile CTAs was slower.
-  // SBGM_B200_MT: 1 = never, 2 = wherever the kernel allows it, unset = by grid size.
   p.mt = 1;
   {
-    static const int mt_mode = [] { const char* e = getenv("SBGM_B200_MT"); return e == nullptr ? 0 : atoi(e); }();
     const bool allowed = planes == 1 && p.ep.staged && proj_w == nullptr && p.splits == 1 && ln_colsum == nullptr && block_n <= 128 &&
                          m_tiles >= 2;
     const long long ctas = static_cast<long long>(m_tiles) * (cout / block_n);
-    if (allowed && mt_mode != 1 && (mt_mode == 2 || ctas >= 252)) p.mt = 2;
+    if (allowed && ctas >= 252) p.mt = 2;
   }
   // Weight multicast over a CTA pair (CL = 2) in slab mode: both CTAs stream the same weight boxes (same output-channel block,
   // same K range), each loads half and multicasts it.  Single-plane activations, staged store, at least one full pair of CTAs
   // along the pixel tiles.  Measured per layer on the C2 forward (profiles/r02_conv_tc_family_table_fp16x2_cluster.txt against
   // ..._mt2_first.txt): the pair runs in lock step, so it pays only where the weight stream is what the layer waits for --
   // 512 -> 512 at 8 x 8: 40.4 -> 36.6 us (478 -> 528 TFLOP/s); the 128- and 256-channel layers are within +-1.5 us either way
-  // (sum over the family 551.6 -> 555.7 us with the pair everywhere).  Default: pairs for cin, cout >= 512 only.
-  // SBGM_B200_CLUSTER: 0 = never, 2 = wherever the kernel allows it, unset = by layer size.
+  // (sum over the family 551.6 -> 555.7 us with the pair everywhere).  Hence pairs for cin, cout >= 512 only.
   p.cluster = 1;
   {
-    static const int cl_mode = [] { const char* e = getenv("SBGM_B200_CLUSTER"); return e == nullptr ? 1 : atoi(e); }();
     const int ctas_x = (m_tiles + p.mt - 1) / p.mt;
     const bool allowed = slab && planes == 1 && p.ep.staged && proj_w == nullptr && ln_colsum == nullptr && block_n <= 128 && ctas_x >= 2;
-    if (allowed && cl_mode != 0 && (cl_mode == 2 || (cin >= 512 && cout >= 512))) p.cluster = 2;
+    if (allowed && cin >= 512 && cout >= 512) p.cluster = 2;
   }
   CUtensorMap ta, tb, to;
   if (slab ? (slab_perm ? encode_perm_map(&ta, in, planes, in_plane, n, h, w, cin, kSlabW, 2, 10)
@@ -887,8 +880,7 @@ static int conv2d_tc_impl(const void* in, size_t in_plane, const void* weight, s
   if (block_n == 128) return launch_conv_tc<SBGM_FMT_BF16X2, 128, 3>(ta, tb, to, p, m_tiles, st);
   // short K loop on a grid of at most one CTA per SM (the attention blocks' Linear layers): four stages put the whole K loop
   // in flight at once -- one TMA round trip instead of two
-  static const bool deep_on = [] { const char* e = getenv("SBGM_B200_DEEP_SHORTK"); return !(e != nullptr && e[0] == '0'); }();
-  if (deep_on && proj_w == nullptr && kh * kw * p.cin_blocks <= 8 && static_cast<long long>(m_tiles) * (cout / 64) * p.splits <= 148)
+  if (proj_w == nullptr && kh * kw * p.cin_blocks <= 8 && static_cast<long long>(m_tiles) * (cout / 64) * p.splits <= 148)
     return launch_conv_tc<SBGM_FMT_BF16X2, 64, 4>(ta, tb, to, p, m_tiles, st);
   return launch_conv_tc<SBGM_FMT_BF16X2, 64, 2>(ta, tb, to, p, m_tiles, st);
 }

@@ -42,17 +42,11 @@ struct WgradCfg {
 __device__ __forceinline__ uint32_t desc_lo_mn(uint32_t addr) { return ((addr & 0x3FFFFu) >> 4) | ((kBoxBytes >> 4) << 16); }
 __device__ __forceinline__ constexpr uint32_t make_idesc_mn(int n) { return make_idesc(n) | (1u << 15) | (1u << 16); }
 
-// CL = CTAs per cluster along x (1 or 2).  The CTAs of a row of the grid (different (tap, channel-block) units, same output
-// channels, same pixel range) all consume the SAME dy tiles: with CL = 2 a pair loads one dy box each (BN = 128: two 64-channel
-// boxes per stage) and multicasts it into both CTAs' stage, halving the dy traffic out of L2.  A stage is released by both
-// consumers (count 2).  An experiment that did not pay (see the launcher): kept opt-in.
-template <int FMT, int BN, int kStages, int CL = 1>
+template <int FMT, int BN, int kStages>
 __global__ void __launch_bounds__(192, 1)
 conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__ CUtensorMap tmap_dy, const WgradParams p) {
   pdl_grid_sync();
   constexpr int kSplit = (FMT == SBGM_FMT_BF16X2) ? 2 : 1;
-  static_assert(CL == 1 || (CL == 2 && kSplit * (BN / 64) == 2), "pairs split the stage's two dy boxes");
-  const uint32_t cta_rank = CL > 1 ? cluster_ctarank() : 0u;
   using Cfg = WgradCfg<kSplit, BN, kStages>;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -69,7 +63,7 @@ conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_co
     tma_prefetch_desc(&tmap_dy);
     for (int s = 0; s < kStages; ++s) {
       mbar_init(full_bar(s), 1);
-      mbar_init(empty_bar(s), CL);
+      mbar_init(empty_bar(s), 1);
     }
     mbar_init(tmem_full_bar, 1);
     fence_barrier_init();
@@ -77,14 +71,11 @@ conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_co
   if (warp == 1) tmem_alloc(tmem_slot, kSplit * BN);
   tcgen05_fence_before();
   __syncthreads();
-  if (CL > 1) cluster_sync_all();
   tcgen05_fence_after();
   const uint32_t tmem_base = *tmem_slot_ptr;
 
-  // a CTA past the last unit pair (the grid is padded to whole clusters) loads its share of dy, computes on unit 0 and stores nothing
-  const bool phantom = static_cast<int>(blockIdx.x) * 2 >= p.units;
-  const int u0 = phantom ? 0 : blockIdx.x * 2;
-  const bool second = !phantom && (u0 + 1) < p.units;
+  const int u0 = blockIdx.x * 2;
+  const bool second = (u0 + 1) < p.units;
   const int u1 = second ? u0 + 1 : u0;
   const int co0 = blockIdx.y * BN;
   const int tile_begin = blockIdx.z * p.tiles_per_split;
@@ -116,15 +107,8 @@ conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_co
             tma_load_5d(a_dst + (pl * 2 + i) * kBoxBytes, &tmap_x, full_bar(stage), cb_[i] * 64, wo0 * p.stride + s_[i] - p.pad,
                         ho0 * p.stride + r_[i] - p.pad, n0, pl);
 #pragma unroll
-          for (int ch = 0; ch < BN / 64; ++ch) {
-            const int box = pl * (BN / 64) + ch;
-            if (CL > 1) {
-              if (box == static_cast<int>(cta_rank))
-                tma_load_5d_multicast(b_dst + box * kBoxBytes, &tmap_dy, full_bar(stage), co0 + ch * 64, wo0, ho0, n0, pl, 0x3);
-            } else {
-              tma_load_5d(b_dst + box * kBoxBytes, &tmap_dy, full_bar(stage), co0 + ch * 64, wo0, ho0, n0, pl);
-            }
-          }
+          for (int ch = 0; ch < BN / 64; ++ch)
+            tma_load_5d(b_dst + (pl * (BN / 64) + ch) * kBoxBytes, &tmap_dy, full_bar(stage), co0 + ch * 64, wo0, ho0, n0, pl);
         }
         if (++stage == kStages) { stage = 0; phase ^= 1u; }
       }
@@ -150,7 +134,7 @@ conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_co
             else umma_bf16_acc(tmem_base, a0 + j * 128, b0 + j * 128, idesc);
           }
         }
-        if (CL > 1) umma_commit_multicast(empty_bar(stage), 0x3); else umma_commit(empty_bar(stage));
+        umma_commit(empty_bar(stage));
         if (tile == tile_end - 1) umma_commit(tmem_full_bar);
         if (++stage == kStages) { stage = 0; phase ^= 1u; }
       }
@@ -160,7 +144,7 @@ conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_co
     const int quarter = warp & 3;
     const int row = quarter * 32 + lane;
     const int unit = (row < 64) ? u0 : u1;
-    const bool valid = !phantom && ((row < 64) || second);
+    const bool valid = (row < 64) || second;
     const size_t kcol = static_cast<size_t>(unit) * 64 + (row & 63);
     float* dst = p.ws + (static_cast<size_t>(blockIdx.z) * p.cout + co0) * p.K + kcol;
     mbar_wait(tmem_full_bar, 0);
@@ -184,7 +168,6 @@ conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_co
   }
   tcgen05_fence_before();
   __syncthreads();
-  if (CL > 1) cluster_sync_all();
   if (warp == 1) tmem_dealloc(tmem_base, kSplit * BN);
 }
 
@@ -331,13 +314,10 @@ static void wgrad_slab_plan(int n, int h, int w, int cin, int cout, WgradSlabPar
 // The slab form pays where a CTA's pixel range is long enough to amortise its 160 KB of partial sums (>= 8 tiles): measured on the
 // C4 step, final conv_up 130 -> 89 us (870 TFLOP/s), the 64 x 64 layers 40 -> 33 us; the 32 x 32 and smaller 64 / 128-channel
 // layers (2-4 tiles per CTA at one or two waves) came out equal or slower and stay on the per-unit kernel.
-// SBGM_B200_WGRAD_SLAB: 0 = never, 2 = wherever the geometry allows, unset = by pixel range.
 static bool wgrad_slab_ok(int fmt, int n, int h, int w, int cin, int cout, int kh, int kw, int stride, int pad) {
-  static const int mode = [] { const char* e = getenv("SBGM_B200_WGRAD_SLAB"); return e == nullptr ? 1 : atoi(e); }();
-  if (mode == 0 || fmt != SBGM_FMT_BF16 || kh != 3 || kw != 3 || stride != 1 || pad != 1 || w % 8 != 0 || h % 16 != 0 || cin % 64 != 0 ||
+  if (fmt != SBGM_FMT_BF16 || kh != 3 || kw != 3 || stride != 1 || pad != 1 || w % 8 != 0 || h % 16 != 0 || cin % 64 != 0 ||
       cout % 64 != 0)
     return false;
-  if (mode == 2) return true;
   WgradSlabParams sp;
   int ss = 0;
   wgrad_slab_plan(n, h, w, cin, cout, &sp, &ss);
@@ -360,9 +340,7 @@ static void wgrad_tc_plan(int n, int ho, int wo, int cin, int cout, int kh, int 
   // the workspace traffic grows with the wave count.  Measured per layer on the C4 step (profiles/r02_wgrad_waves_*.txt): the
   // 64-wide layers (few CTAs per pixel range, long pixel ranges) are faster with three waves (final conv_up 130 vs 205 us), the
   // 128-wide ones (many (tap, channel-block) units) with one (36 launches: 362 vs 462 us, and a third of the reduce traffic).
-  // SBGM_B200_WGRAD_WAVES overrides both.
-  static const int forced = [] { const char* e = getenv("SBGM_B200_WGRAD_WAVES"); const int v = e ? atoi(e) : 0; return v >= 1 && v <= 8 ? v : 0; }();
-  const int waves = forced ? forced : (*bn == 64 ? 3 : 1);
+  const int waves = *bn == 64 ? 3 : 1;
   int s = (148 * waves + base - 1) / base;
   if (s > p->total_tiles) s = p->total_tiles;
   if (s < 1) s = 1;
@@ -370,11 +348,11 @@ static void wgrad_tc_plan(int n, int ho, int wo, int cin, int cout, int kh, int 
   *splits = (p->total_tiles + p->tiles_per_split - 1) / p->tiles_per_split;
 }
 
-template <int FMT, int BN, int kStages, int CL = 1>
+template <int FMT, int BN, int kStages>
 static int launch_wgrad_tc(const CUtensorMap& tx, const CUtensorMap& td, const WgradParams& p, int splits, cudaStream_t st) {
   constexpr int kSplit = (FMT == SBGM_FMT_BF16X2) ? 2 : 1;
   using Cfg = WgradCfg<kSplit, BN, kStages>;
-  auto kern = conv_wgrad_tc_kernel<FMT, BN, kStages, CL>;
+  auto kern = conv_wgrad_tc_kernel<FMT, BN, kStages>;
   static bool configured = false;
   if (!configured) {
     if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes) != cudaSuccess) {
@@ -383,13 +361,7 @@ static int launch_wgrad_tc(const CUtensorMap& tx, const CUtensorMap& td, const W
     }
     configured = true;
   }
-  dim3 grid((p.units + 1) / 2, p.cout / BN, splits);
-  if (CL > 1) {
-    grid.x = (grid.x + CL - 1) / CL * CL;
-    launch_k_cluster((kern), grid, 192, Cfg::kSmemBytes, st, CL, tx, td, p);
-  } else {
-    launch_k((kern), grid, 192, Cfg::kSmemBytes, st, tx, td, p);
-  }
+  launch_k((kern), dim3((p.units + 1) / 2, p.cout / BN, splits), 192, Cfg::kSmemBytes, st, tx, td, p);
   return check_launch("conv2d_wgrad_tc");
 }
 
@@ -414,28 +386,13 @@ extern "C" size_t sbgm_conv2d_wgrad_tc_workspace_floats(int fmt, int n, int h, i
   return static_cast<size_t>(splits) * cout * p.K;
 }
 
-extern "C" int sbgm_conv2d_wgrad_tc_splits(int fmt, int n, int h, int w, int cin, int cout, int kh, int kw, int stride, int pad) {
-  if (cin % 64 != 0 || cout % 64 != 0 || stride < 1) return 0;
-  const int ho = (h + 2 * pad - kh) / stride + 1, wo = (w + 2 * pad - kw) / stride + 1;
-  if (ho <= 0 || wo <= 0) return 0;
-  if (wgrad_slab_ok(fmt, n, h, w, cin, cout, kh, kw, stride, pad)) {
-    WgradSlabParams sp;
-    int ss = 0;
-    wgrad_slab_plan(n, h, w, cin, cout, &sp, &ss);
-    return ss;
-  }
-  WgradParams p;
-  int bn = 0, splits = 0;
-  wgrad_tc_plan(n, ho, wo, cin, cout, kh, kw, fmt, &p, &bn, &splits);
-  return splits;
-}
-
 extern "C" int sbgm_conv2d_wgrad_tc(const void* x, size_t x_plane, const void* dy, size_t dy_plane, float* dweight_oihw, int fmt,
                                     int n, int h, int w, int cin, int cout, int kh, int kw, int stride, int pad, float* workspace,
                                     void* stream) {
   SBGM_REQUIRE(fmt == SBGM_FMT_BF16 || fmt == SBGM_FMT_BF16X2, "conv2d_wgrad_tc: format %d is not a tensor-core format", fmt);
   SBGM_REQUIRE(cin % 64 == 0 && cout % 64 == 0, "conv2d_wgrad_tc: cin=%d and cout=%d must be multiples of 64", cin, cout);
   SBGM_REQUIRE(stride >= 1 && stride <= 8, "conv2d_wgrad_tc: stride %d unsupported", stride);
+  SBGM_REQUIRE(dweight_oihw != nullptr, "conv2d_wgrad_tc: dweight_oihw is required");
   const int ho = (h + 2 * pad - kh) / stride + 1, wo = (w + 2 * pad - kw) / stride + 1;
   SBGM_REQUIRE(ho > 0 && wo > 0, "conv2d_wgrad_tc: empty output");
   const int planes = (fmt == SBGM_FMT_BF16X2) ? 2 : 1;
@@ -457,7 +414,6 @@ extern "C" int sbgm_conv2d_wgrad_tc(const void* x, size_t x_plane, const void* d
     }
     launch_k((conv_wgrad_slab_kernel), dim3(sp.cin_blocks, cout / 64, ss), 192, kWsSmemBytes, as_stream(stream), sx, sd, sp);
     if (check_launch("conv2d_wgrad_tc")) return 1;
-    if (dweight_oihw == nullptr) return 0;
     return sbgm_wgrad_reduce(workspace, ss, cout, 9, cin, dweight_oihw, stream);
   }
   WgradParams p;
@@ -470,16 +426,9 @@ extern "C" int sbgm_conv2d_wgrad_tc(const void* x, size_t x_plane, const void* d
   if (encode_act_map(&td, dy, planes, dy_plane, n, ho, wo, cout, p.w_tile, p.h_tile, p.n_tile, 1)) return 1;
   cudaStream_t st = as_stream(stream);
   int rc;
-  // dy multicast over CTA pairs where a stage holds two dy boxes and there are at least two unit pairs.  Measured SLOWER on the C4
-  // step (30 paired launches 407 us + 6 unpaired 34 us against 364 us for the 36 unpaired; step 5.78 vs 5.66-5.77 ms): the pair
-  // runs in lock step and the kernel is not waiting for L2 bandwidth.  Opt-in: SBGM_B200_WGRAD_CLUSTER=1.
-  static const bool pairs_on = [] { const char* e = getenv("SBGM_B200_WGRAD_CLUSTER"); return e != nullptr && e[0] == '1'; }();
-  const bool pairs = pairs_on && p.units >= 3;
-  if (fmt == SBGM_FMT_BF16) rc = (bn == 128) ? (pairs ? launch_wgrad_tc<SBGM_FMT_BF16, 128, 3, 2>(tx, td, p, splits, st)
-                                                      : launch_wgrad_tc<SBGM_FMT_BF16, 128, 3>(tx, td, p, splits, st))
+  if (fmt == SBGM_FMT_BF16) rc = (bn == 128) ? launch_wgrad_tc<SBGM_FMT_BF16, 128, 3>(tx, td, p, splits, st)
                                              : launch_wgrad_tc<SBGM_FMT_BF16, 64, 4>(tx, td, p, splits, st);
-  else rc = pairs ? launch_wgrad_tc<SBGM_FMT_BF16X2, 64, 2, 2>(tx, td, p, splits, st) : launch_wgrad_tc<SBGM_FMT_BF16X2, 64, 2>(tx, td, p, splits, st);
+  else rc = launch_wgrad_tc<SBGM_FMT_BF16X2, 64, 2>(tx, td, p, splits, st);
   if (rc) return rc;
-  if (dweight_oihw == nullptr) return 0;      // the caller sums the slabs later (sbgm_wgrad_reduce_batch)
   return sbgm_wgrad_reduce(workspace, splits, cout, kh * kw, cin, dweight_oihw, stream);
 }

@@ -523,8 +523,7 @@ int resident_blocks(const void* kern, int block, size_t smem) {
   if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, block, smem) != cudaSuccess || per_sm < 1) per_sm = 4;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  static const bool on = [] { const char* e = getenv("SBGM_B200_WAVE_GRID"); return !(e != nullptr && e[0] == '0'); }();
-  const int v = on ? per_sm * sms : 148 * 8;
+  const int v = per_sm * sms;
   cache[kern] = v;
   return v;
 }

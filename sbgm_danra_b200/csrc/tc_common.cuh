@@ -57,13 +57,6 @@ __device__ __forceinline__ void tma_load_3d_multicast(uint32_t dst, const CUtens
       ::"r"(dst), "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "h"(cta_mask)
       : "memory");
 }
-__device__ __forceinline__ void tma_load_5d_multicast(uint32_t dst, const CUtensorMap* map, uint32_t bar, int c0, int c1, int c2, int c3, int c4,
-                                                      uint16_t cta_mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.5d.shared::cluster.global.tile.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4, %5, %6, %7}], [%2], %8;"
-      ::"r"(dst), "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4), "h"(cta_mask)
-      : "memory");
-}
 __device__ __forceinline__ uint32_t cluster_ctarank() {
   uint32_t r;
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));

@@ -47,10 +47,7 @@ def _stream() -> int:
 # the launch sequence so that its in-graph cost can be read off as a difference.  Results are garbage when set.
 import os as _os
 _SKIP = frozenset(x for x in _os.environ.get("SBGM_B200_SKIP", "").split(",") if x)
-_STEM_FUSED = _os.environ.get("SBGM_B200_STEM_FUSED", "1") != "0"     # 0: stem as im2col tensor + 1x1 convolution
-_LN_FOLD = _os.environ.get("SBGM_B200_LN_FOLD", "1") != "0"           # 0: LayerNorm as its own kernel in front of in_proj / ff.0
 _UP_FUSED = _os.environ.get("SBGM_B200_UP_FUSED", "1") != "0"         # 0: the bilinear upsample ahead of a 64 -> 64 conv_up as its own launch
-_ATTN_FUSED = _os.environ.get("SBGM_B200_ATTN_FUSED", "auto")         # 0: attention core and out-projection as two launches
 
 
 # Measurement hook (bench.py `roofline.family`): when set to a list, every convolution / Linear launch of a forward appends
@@ -282,15 +279,6 @@ class Kernels:
              out.ptr, out.plane, self.fmt, n, h, w, _stream())
         return out
 
-    def conv1x1_bcast(self, x: Act, cw: ConvW, residual: Act, tproj: Optional[torch.Tensor]) -> Act:
-        """1x1 tensor-core convolution whose residual may be a single image broadcast over the batch."""
-        out = Act(self.fmt, x.n, x.h, x.w, cw.cout, self.device)
-        mod = x.h * x.w if (residual.n == 1 and x.n > 1) else 0
-        call("sbgm_conv2d_tc_ex", x.ptr, x.plane, cw.w.data_ptr(), cw.plane, _ptr(cw.bias), residual.ptr, residual.plane, mod,
-             _ptr(tproj), tproj.stride(0) if tproj is not None else 0, out.ptr, out.plane, self.fmt, x.n, x.h, x.w, cw.cin, cw.cout,
-             1, 1, 1, 0, 0, x.h, x.w, x.h, x.w, 1, 0, 0, ACT_NONE, None, 0, _stream())
-        return out
-
     def linear(self, x: Act, cw: ConvW, act: int = ACT_NONE, residual: Optional[Act] = None) -> Act:
         return self.conv(x, cw, 1, 0, act, residual)
 
@@ -382,14 +370,12 @@ class Kernels:
         return out
 
     def attention_out_proj_ok(self, b: int, s: int, c: int, heads: int) -> bool:
-        """True if the attention core + out-projection + residual run as one tcgen05 kernel (csrc/attn_fused.cu).
-        SBGM_B200_ATTN_FUSED: 0 = never, 1 = wherever the kernel supports the shape, unset = where it measured faster than the
-        two launches it replaces: enough query tiles to fill the GPU (16 x 16 maps at the benchmark batch)."""
-        if _ATTN_FUSED == "0" or "attn_core" in _SKIP:
+        """True if the attention core + out-projection + residual run as one tcgen05 kernel (csrc/attn_fused.cu): where the
+        kernel supports the shape and it measured faster than the two launches it replaces, i.e. with enough query tiles to fill
+        the GPU (16 x 16 maps at the benchmark batch)."""
+        if "attn_core" in _SKIP or not _lib.query("sbgm_attention_out_proj_supported", self.fmt, b, s, c, heads):
             return False
-        if not _lib.query("sbgm_attention_out_proj_supported", self.fmt, b, s, c, heads):
-            return False
-        return _ATTN_FUSED == "1" or b * s >= 128 * 96
+        return b * s >= 128 * 96
 
     def attention_out_proj(self, qkv: Act, x: Act, cw: ConvW, b: int, s: int, c: int, heads: int) -> Act:
         """x + out_proj(softmax(Q K^T / sqrt(d)) V): scores, probabilities and head outputs stay on the SM."""
@@ -416,7 +402,7 @@ class AttentionW:
         self.ff0 = pk.conv(f"{prefix}.ff.0.weight", f"{prefix}.ff.0.bias")
         self.ff2 = pk.conv(f"{prefix}.ff.2.weight", f"{prefix}.ff.2.bias")
         # LayerNorm folded into the Linear layer behind it (tensor-core formats): ln1 -> in_proj, ln2 -> ff.0
-        self.fold = pk.fmt != FMT_F32 and _LN_FOLD
+        self.fold = pk.fmt != FMT_F32
         if self.fold:
             self.in_proj_ln = pack_linear_ln(pk, f"{prefix}.mha.in_proj_weight", f"{prefix}.mha.in_proj_bias", f"{prefix}.ln1.weight",
                                              f"{prefix}.ln1.bias")
@@ -565,15 +551,14 @@ class EncoderEngine:
         t0 = tp.cols(tproj, "enc0")
         if self.fmt != FMT_F32:
             # conv1 on the tensor cores: im2col of the 8x8 stride-2 window, then a 1x1 implicit GEMM (K = 64 per channel)
-            if (partial is not None or cc == 0) and _STEM_FUSED and h % 16 == 0 and w % 32 == 0:
+            if (partial is not None or cc == 0) and h % 16 == 0 and w % 32 == 0:
                 # one kernel: windows of x built in shared memory, MMA against the resident 64 x 64 weights, + partial + time
                 f1 = Act(self.fmt, n, h // 2, w // 2, 64, self.device)
                 call("sbgm_stem_x_tc", x.data_ptr(), self.stem_cw_x.w.data_ptr(), self.stem_cw_x.plane,
                      None if partial is None else partial.ptr, 0 if partial is None else partial.plane, 0 if partial is None else partial.n,
                      t0.data_ptr(), t0.stride(0), f1.ptr, f1.plane, self.fmt, n, h, w, _stream())
-            elif partial is not None:
-                f1 = k.conv1x1_bcast(k.stem_im2col(x, None, 0, 1, cc), self.stem_cw_x, partial, t0)
             else:
+                assert partial is None, f"a precomputed stem partial needs h % 16 == 0 and w % 32 == 0, got {h} x {w}"
                 if cc > 0:
                     assert planes is not None and planes.shape[1] == cc, f"encoder expects {cc} conditioning channels"
                 f1 = k.conv(k.stem_im2col(x, planes, 0, self.cin, cc), self.stem_cw_all, tproj=t0)

@@ -156,9 +156,8 @@ class _NativeStep:
     """One fused sampler step on the engine, written so it can be captured in a CUDA graph.  All buffers have
     fixed addresses; a new sampler call with the same shapes only rewrites their contents."""
 
-    def __init__(self, model, batch: int, size: int, n_steps: int, has_y: bool, planes_batch: int, cfg_scale: Optional[float],
-                 lane: int = 0):
-        eng = model.engine(lane)
+    def __init__(self, model, batch: int, size: int, n_steps: int, has_y: bool, planes_batch: int, cfg_scale: Optional[float]):
+        eng = model.engine()
         self.eng, self.dev, self.b, self.size = eng, eng.device, batch, size
         dev = self.dev
         self.table = torch.zeros((n_steps, STEP_COLS), dtype=torch.float32, device=dev)
@@ -398,12 +397,6 @@ def _sample(kind: str, score_model, marginal_prob_std, diffusion_coeff, batch_si
     sharded = kind == "pc" and _state.members_total is not None and _state.members_total != batch_size
     total = _state.members_total if sharded else batch_size
 
-    lanes = int(os.environ.get("SBGM_B200_LANES", "1"))
-    if (native and use_graph and kind == "em" and lanes == 2 and n_steps > 1 and batch_size >= 16 and batch_size % 2 == 0
-            and not score_model.training):
-        return _sample_em_two_lanes(score_model, table, seed, scale, dev, batch_size, n_steps, img_size, std1, first_elem,
-                                    y, cond_img, lsm_cond, topo_cond)
-
     with torch.no_grad(), torch.cuda.device(dev):
         if native:
             eng = score_model.engine()
@@ -478,77 +471,6 @@ def _sample(kind: str, score_model, marginal_prob_std, diffusion_coeff, batch_si
                     st.k = k
                 one_step()
         return st.mean.clone()
-
-
-def _sample_em_two_lanes(score_model, table, seed, scale, dev, batch_size, n_steps, img_size, std1, first_elem, y, cond_img,
-                         lsm_cond, topo_cond) -> torch.Tensor:
-    """Euler-Maruyama with the ensemble split into two half-batches that run on two streams inside ONE captured graph
-    (SBGM_B200_LANES=2).  The members are independent, the Philox stream is keyed by the global element index, so the result is
-    the one-lane result bit for bit; the point is overlap: the launch/latency-bound kernels of one lane (the attention blocks'
-    Linear layers, the 4x4 / 8x8 maps) run in the shadow of the other lane's throughput-bound convolutions.  Each lane owns an
-    engine (packed weights, split-K / statistics scratch) and its activation buffers."""
-    half = batch_size // 2
-    per = img_size * img_size
-    with torch.no_grad(), torch.cuda.device(dev):
-        eng0 = score_model.engine(0)
-        planes = _NativeStep.planes_of(eng0, batch_size, cond_img, lsm_cond, topo_cond)
-        planes_u = None
-        if scale is not None and planes is not None:
-            planes_u = _NativeStep.planes_of(eng0, batch_size, None if cond_img is None else torch.zeros_like(cond_img),
-                                             _strip_mask(lsm_cond), _strip_mask(topo_cond))
-            if planes_u.shape[0] != planes.shape[0]:
-                planes_u = planes_u.expand(planes.shape[0], -1, -1, -1).contiguous()
-        pb = 0 if planes is None else planes.shape[0]
-        key = ("lanes2", id(eng0), id(score_model.engine(1)), batch_size, img_size, n_steps, scale, y is not None, pb, first_elem)
-        plan = next((p for k, p in _PLAN_CACHE if k == key), None)
-        if plan is None:
-            with torch.inference_mode(False):
-                plan = [_NativeStep(score_model, half, img_size, n_steps, y is not None, min(pb, half) if pb > 1 else pb, scale,
-                                    lane=l) for l in range(2)]
-            plan.append({"graph": None, "per_replay": 0, "streams": [torch.cuda.Stream(device=dev) for _ in range(2)]})
-            _PLAN_CACHE.insert(0, (key, plan))
-            del _PLAN_CACHE[_PLAN_CACHE_SIZE:]
-        st2, meta = plan[:2], plan[2]
-
-        def cut(v, l):
-            return None if v is None else (v if v.shape[0] == 1 else v[l * half:(l + 1) * half].contiguous())
-
-        for l, st in enumerate(st2):
-            st.load(table, seed, None if y is None else y.reshape(-1)[l * half:(l + 1) * half], cut(planes, l), cut(planes_u, l))
-
-        def one_step(l: int) -> None:
-            st2[l].score_into()
-            _predict(st2[l], 1, 1, first_elem + l * half * per)
-
-        def both(capturing: bool) -> None:
-            cur = torch.cuda.current_stream(dev)
-            for l, sd_ in enumerate(meta["streams"]):
-                sd_.wait_stream(cur)
-                with torch.cuda.stream(sd_):
-                    one_step(l)
-            for sd_ in meta["streams"]:
-                cur.wait_stream(sd_)
-
-        if meta["graph"] is None:
-            side = torch.cuda.Stream(device=dev)
-            side.wait_stream(torch.cuda.current_stream(dev))
-            with torch.cuda.stream(side):
-                both(False)                                   # eager warm-up (lazy kernel attributes, scratch buffers)
-            torch.cuda.current_stream(dev).wait_stream(side)
-            torch.cuda.synchronize(dev)
-            meta["graph"] = torch.cuda.CUDAGraph()
-            before = _lib_stats.launches
-            with graph_capture(meta["graph"]):
-                both(True)
-            meta["per_replay"] = _lib_stats.launches - before
-            _lib_stats.launches = before
-        for l, st in enumerate(st2):
-            st.counter[:2].zero_()
-            call("sbgm_sampler_init", st.x.data_ptr(), st.x.numel(), std1, seed, first_elem + l * half * per, _eng._stream())
-        for _ in range(n_steps):
-            meta["graph"].replay()
-            _lib_stats.launches += meta["per_replay"]
-        return torch.cat([st2[0].mean, st2[1].mean], dim=0)
 
 
 def Euler_Maruyama_sampler(score_model, marginal_prob_std, diffusion_coeff, batch_size=64, num_steps=500,

@@ -425,15 +425,13 @@ class ScoreNet(nn.Module):
                              out_channels=d.output_channels, use_resize_conv=d.use_resize_conv, norm=d.norm,
                              gn_groups=d.gn_groups, activation=_act_name(d.activation))
 
-    def engine(self, lane: int = 0) -> _eng.UNetEngine:
-        """Packed-weight engine for the current parameters (cached; rebuilt after parameter updates).  `lane` > 0 gives an
-        independent engine (own packed weights and scratch buffers) for a second concurrent stream of the samplers."""
+    def engine(self) -> _eng.UNetEngine:
+        """Packed-weight engine for the current parameters (cached; rebuilt after parameter updates)."""
         _require_cuda(self.encoder.conv1.weight, "ScoreNet")
-        cache = self._cache if lane == 0 else self.__dict__.setdefault("_lane_caches", {}).setdefault(lane, _EngineCache())
-        return cache.get(self, self.precision, lambda dev: _eng.UNetEngine(self.state_dict(), self.spec(), self.precision, dev))
+        return self._cache.get(self, self.precision, lambda dev: _eng.UNetEngine(self.state_dict(), self.spec(), self.precision, dev))
 
     # derived device state (packed weights, captured CUDA graphs, gradient exchange): never copied or pickled with the model
-    _DERIVED = ("_cache", "_lane_caches", "_train_runners", "_grad_sync", "_members")
+    _DERIVED = ("_cache", "_train_runners", "_grad_sync", "_members")
 
     def __deepcopy__(self, memo):
         """`copy.deepcopy(model)` (the reference's EMA copy, sbgm/training.py:114) copies parameters and buffers only; the copy

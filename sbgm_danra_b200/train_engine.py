@@ -14,7 +14,6 @@ torch supplies memory, streams and the autograd hook; every FLOP runs in this re
 from __future__ import annotations
 
 import ctypes
-import os
 from typing import Callable, Dict, List, Optional, Sequence, Tuple
 
 import torch
@@ -199,50 +198,17 @@ class Tape:
             call("sbgm_add_inplace", cur.ptr, cur.plane, g.ptr, g.plane, self.fmt, cur.plane, _stream())
 
 
-class _ReduceJob(ctypes.Structure):      # mirrors sbgm_wgrad_reduce_job (include/sbgm_b200.h)
-    _fields_ = [("workspace", ctypes.c_void_p), ("dweight_oihw", ctypes.c_void_p), ("splits", ctypes.c_int), ("cout", ctypes.c_int),
-                ("taps", ctypes.c_int), ("cin", ctypes.c_int)]
-
-
-# Deferred / batched split reduction of the weight gradients: measured neutral on the C4 step (46 reduce launches -> 5, kernel
-# time -0.03 ms, wall time +-0 within noise: 5.67-5.69 vs 5.66 ms; kernel boundaries inside a graph overlap, profiles/
-# r02_train_step_graph_gaps.txt), and it delays the gradients' readiness for the bucketed all-reduce -> opt-in.
-_WGRAD_BATCH = os.environ.get("SBGM_B200_WGRAD_BATCH", "0") == "1"
-_WGRAD_FLUSH_ELEMS = int(os.environ.get("SBGM_B200_WGRAD_FLUSH_ELEMS", str(3 << 20)))     # gradients per batched reduce (elements)
-
-
 class TrainKernels:
     """Forward ops that record their backward on a tape."""
 
-    def __init__(self, fmt: int, device, flat_grad: Callable[[str, Tuple[int, ...]], torch.Tensor],
-                 flat_view: Optional[Callable[[str, Tuple[int, ...]], torch.Tensor]] = None,
-                 on_ready: Optional[Callable[[List[str]], None]] = None) -> None:
-        """`flat_grad(name, shape)`: the gradient view of a parameter, reported as produced at once.  With `flat_view` (the same
-        view, not reported) and `on_ready(names)` the tensor-core weight gradients are DEFERRED: the kernel leaves its split
-        slabs in a workspace and `flush_wgrad` sums the slabs of several layers in one launch, then reports them."""
+    def __init__(self, fmt: int, device, flat_grad: Callable[[str, Tuple[int, ...]], torch.Tensor]) -> None:
+        """`flat_grad(name, shape)`: the gradient view of a parameter, reported as produced at once."""
         self.fmt, self.device = fmt, device
         self.k = Kernels(fmt, device)
         self.tape: Optional[Tape] = None
         self.param_grad = flat_grad
-        self.param_view, self.on_ready = flat_view, on_ready
-        self.pending: List[Tuple[torch.Tensor, torch.Tensor, int, int, int, int, str]] = []
-        self.pending_elems = 0
         self.sync_bn = None          # torch.distributed process group: synchronise BatchNorm statistics over it
         self._scratch: Dict[str, torch.Tensor] = {}
-
-    def flush_wgrad(self) -> None:
-        """Sum the split slabs of every deferred weight gradient (one launch) and report the gradients as produced."""
-        if not self.pending:
-            return
-        jobs = (_ReduceJob * len(self.pending))()
-        for k, (ws, dw, splits, cout, taps, cin, _) in enumerate(self.pending):
-            jobs[k].workspace, jobs[k].dweight_oihw = ws.data_ptr(), dw.data_ptr()
-            jobs[k].splits, jobs[k].cout, jobs[k].taps, jobs[k].cin = splits, cout, taps, cin
-        call("sbgm_wgrad_reduce_batch", jobs, len(self.pending), _stream())
-        names = [p[6] for p in self.pending]
-        self.pending, self.pending_elems = [], 0
-        if self.on_ready is not None:
-            self.on_ready(names)
 
     # -- scratch management --------------------------------------------------------------------
     TICKET_WORDS = 4096        # leading words of a ticketed scratch buffer (kNormTicketWords / kChansumTicketWords)
@@ -308,18 +274,7 @@ class TrainKernels:
             ws = self.scratch("chansum", _lib.query("sbgm_channel_sums_scratch_floats", dy.n, cout), tickets=True)
             call("sbgm_channel_sums", dy.ptr, dy.plane, fmt, dy.n, dy.h * dy.w, cout, None, 0, db.data_ptr(), ws.data_ptr(), st)
         tc = fmt != FMT_F32 and cin % 64 == 0 and cout % 64 == 0
-        if tc and self.param_view is not None:
-            # deferred: the split slabs stay in their own workspace until flush_wgrad sums several layers' worth in one launch
-            dw = self.param_view(layer.name, layer.shape)
-            geo = (fmt, n, h, w, cin, cout, kh, kw, stride, pad)
-            ws = torch.empty(_lib.query("sbgm_conv2d_wgrad_tc_workspace_floats", *geo), dtype=torch.float32, device=self.device)
-            call("sbgm_conv2d_wgrad_tc", x.ptr, x.plane, dy.ptr, dy.plane, None, fmt, n, h, w, cin, cout, kh, kw, stride, pad,
-                 ws.data_ptr(), st)
-            self.pending.append((ws, dw, _lib.query("sbgm_conv2d_wgrad_tc_splits", *geo), cout, kh * kw, cin, layer.name))
-            self.pending_elems += dw.numel()
-            if self.pending_elems >= _WGRAD_FLUSH_ELEMS or len(self.pending) >= 48:
-                self.flush_wgrad()
-        elif tc:
+        if tc:
             dw = self.param_grad(layer.name, layer.shape)
             ws = self.scratch("wgrad", _lib.query("sbgm_conv2d_wgrad_tc_workspace_floats", fmt, n, h, w, cin, cout, kh, kw, stride, pad))
             call("sbgm_conv2d_wgrad_tc", x.ptr, x.plane, dy.ptr, dy.plane, dw.data_ptr(), fmt, n, h, w, cin, cout, kh, kw, stride, pad,
@@ -629,7 +584,7 @@ class TrainEngine:
         self.flat_numel = off
         self.flat: Optional[torch.Tensor] = None
         self.touched: Dict[str, torch.Tensor] = {}
-        self.tk = TrainKernels(self.fmt, device, self._param_grad, *((self._param_view, self._grads_ready) if _WGRAD_BATCH else ()))
+        self.tk = TrainKernels(self.fmt, device, self._param_grad)
         self.grad_sync = None      # parallel.GradSync or None
         with torch.cuda.device(device), torch.no_grad():
             self._pack()
@@ -640,16 +595,6 @@ class TrainEngine:
         g = self.flat[off:off + numel].view(shape)
         self.touched[name] = g
         return g
-
-    def _param_view(self, name: str, shape: Tuple[int, ...]) -> torch.Tensor:
-        """The gradient view without reporting it (deferred weight gradients: reported by `_grads_ready` once reduced)."""
-        off, numel = self.offsets[name]
-        return self.flat[off:off + numel].view(shape)
-
-    def _grads_ready(self, names: List[str]) -> None:
-        for name in names:
-            off, numel = self.offsets[name]
-            self.touched[name] = self.flat[off:off + numel].view(tuple(self.sd[name].shape))
 
     def _bn(self, prefix: str) -> dict:
         return dict(weight=self.sd[f"{prefix}.weight"], bias=self.sd[f"{prefix}.bias"], running_mean=self.sd[f"{prefix}.running_mean"],
@@ -884,10 +829,6 @@ class TrainEngine:
                 new = list(self.touched)[reported:]
                 reported = len(self.touched)
                 sync.progress(new)
-        tk.flush_wgrad()
-        if sync is not None and len(self.touched) > reported:
-            sync.progress(list(self.touched)[reported:])
-            reported = len(self.touched)
         # time embedding: one launch set for all nine projections (+ label embedding)
         fw, pw, pb, ps = self.tp._packed
         rows = t.numel()

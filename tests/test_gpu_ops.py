@@ -555,9 +555,7 @@ def test_stem_fused_window_kernel(E, prec, n, size, bcast, with_partial):
 ], ids=lambda c: "x".join(map(str, c)))
 def test_conv2d_two_pixel_tiles_per_cta(E, prec, case, monkeypatch):
     """The MT = 2 kernels (two 128-pixel tiles per CTA sharing every weight box) against torch, with the fused GroupNorm statistics
-    where the layer has them; forced on with SBGM_B200_MT=2 is not possible inside one process (the switch is read once), so
-    the cases are shapes the automatic choice sends to MT = 2 -- checked through equality with the one-tile result of a
-    fresh process in test_mt_switch_equivalence."""
+    where the layer has them.  The cases are shapes that the grid-size rule (>= 252 one-tile CTAs) sends to MT = 2."""
     n, h, w, cin, cout, k, stride, pad, epi = case
     fmt = FMTS[prec]
     x = gen(n, cin, h, w, seed=1)

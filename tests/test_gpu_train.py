@@ -844,37 +844,6 @@ def test_channel_sums(E, prec, n, hw, c, per_sample):
     assert int(ws[:4096].view(torch.int32).abs().sum()) == 0
 
 
-def test_deferred_weight_gradients_equal_immediate_ones(E, T):
-    """TrainKernels with a `flat_view`: the tensor-core weight gradients leave their split slabs in workspaces and ONE batched
-    reduce (sbgm_wgrad_reduce_batch) finishes several layers; bit-identical to the per-layer reduce, reported only at the flush."""
-    fmt = FMTS["bf16"]
-    cases = [(2, 16, 16, 64, 64, 3, 1, 1), (2, 8, 8, 128, 256, 3, 1, 1), (1, 1, 300, 256, 768, 1, 1, 0), (2, 16, 16, 64, 128, 3, 2, 1)]
-    results = []
-    for deferred in (False, True):
-        grads, ready = {}, []
-
-        def view(name, shape):
-            if name not in grads:
-                grads[name] = torch.zeros(shape, dtype=torch.float32, device=DEV)
-            return grads[name]
-
-        tk = T.TrainKernels(fmt, torch.device(DEV), view, view if deferred else None, ready.extend if deferred else None)
-        tk.tape = T.Tape(fmt, torch.device(DEV))
-        for k, (n, h, w, cin, cout, ks, stride, pad) in enumerate(cases):
-            layer = T.ConvLayer(f"w{k}", gen(cout, cin, ks, ks, seed=k).to(DEV), None, fmt)
-            xa = act_of(E, gen(n, cin, h, w, seed=10 + k), fmt)
-            ya = tk.conv(xa, layer, stride=stride, pad=pad, need_dx=False)
-            tk.tape.add(ya, act_of(E, gen(n, cout, ya.h, ya.w, seed=20 + k), fmt))
-        run_tape(tk)
-        if deferred:
-            assert ready == [] and len(tk.pending) == len(cases)            # nothing reported before the flush
-            tk.flush_wgrad()
-            assert sorted(ready) == sorted(grads) and tk.pending == []
-        results.append({k: v.clone() for k, v in grads.items()})
-    for k in results[0]:
-        assert torch.equal(results[0][k], results[1][k]), k
-
-
 def test_graph_capture_survives_a_pinning_thread():
     """The training graphs are captured on the third step, while a DataLoader(pin_memory=True) thread may be allocating pinned
     memory and querying events: the capture must not be invalidated by CUDA calls of OTHER threads (capture_error_mode)."""

@@ -167,11 +167,10 @@ def test_deepcopy_and_pickle_leave_device_caches_behind():
     net.precision = "bf16"
     net._cache.key, net._cache.value = "k", threading.Lock()            # stand-ins for engines / CUDA graphs
     net.__dict__["_train_runners"] = {"cfg": threading.Lock()}
-    net.__dict__["_lane_caches"] = {1: threading.Lock()}
     net._grad_sync = threading.Lock()
     for twin in (copy.deepcopy(net), pickle.loads(pickle.dumps(net))):
         assert twin._cache is not net._cache and twin._cache.key is None and twin._cache.value is None
-        assert "_train_runners" not in twin.__dict__ and "_lane_caches" not in twin.__dict__
+        assert "_train_runners" not in twin.__dict__
         assert getattr(twin, "_grad_sync", None) is None and twin.precision == "bf16"
         assert twin.debug_pre_sigma_div == net.debug_pre_sigma_div and twin.training == net.training
         a, b = net.state_dict(), twin.state_dict()

@@ -20,7 +20,7 @@ Precisions
 from __future__ import annotations
 
 from dataclasses import dataclass
-from typing import Dict, List, Optional, Sequence, Tuple
+from typing import Callable, Dict, List, NamedTuple, Optional, Sequence, Tuple
 
 import torch
 
@@ -47,7 +47,6 @@ def _stream() -> int:
 # the launch sequence so that its in-graph cost can be read off as a difference.  Results are garbage when set.
 import os as _os
 _SKIP = frozenset(x for x in _os.environ.get("SBGM_B200_SKIP", "").split(",") if x)
-_UP_FUSED = _os.environ.get("SBGM_B200_UP_FUSED", "1") != "0"         # 0: the bilinear upsample ahead of a 64 -> 64 conv_up as its own launch
 
 
 # Measurement hook (bench.py `roofline.family`): when set to a list, every convolution / Linear launch of a forward appends
@@ -78,11 +77,15 @@ class Act:
     def ptr(self) -> int:
         return self.buf.data_ptr()
 
+    def view(self, n: int, h: int, w: int, c: int) -> "Act":
+        """The same storage as an [n, h, w, c] tensor of the same size (no copy)."""
+        v = Act.__new__(Act)
+        v.buf, v.fmt, v.n, v.h, v.w, v.c = self.buf, self.fmt, n, h, w, c
+        return v
+
     def tokens(self) -> "Act":
         """View [n, h, w, c] as a token matrix [1, 1, n*h*w, c] (no copy)."""
-        v = Act.__new__(Act)
-        v.buf, v.fmt, v.n, v.h, v.w, v.c = self.buf, self.fmt, 1, 1, self.n * self.h * self.w, self.c
-        return v
+        return self.view(1, 1, self.n * self.h * self.w, self.c)
 
     def like(self, c: Optional[int] = None, h: Optional[int] = None, w: Optional[int] = None) -> "Act":
         return Act(self.fmt, self.n, h or self.h, w or self.w, c or self.c, self.buf.device)
@@ -115,6 +118,39 @@ class ConvW:
     @property
     def plane(self) -> int:
         return self.cout * self.kh * self.kw * self.cin
+
+
+@dataclass
+class TransposeW:
+    """A packed nn.ConvTranspose2d(cin, cout, kernel 2, stride 2) (score_unet.py:466-468, the use_resize_conv=False decoder):
+    out[n, 2i+a, 2j+b, co] = bias[co] + sum_ci x[n, i, j, ci] W[ci][co][a][b] -- four 1x1 convolutions scattered to the four
+    output parities (`subs`: (a, b, ConvW), tensor cores), or one gather over the 2x2 taps (`simt` [4][cin][cout], fp32)."""
+    bias: torch.Tensor
+    cin: int
+    cout: int
+    simt: Optional[torch.Tensor] = None
+    subs: Optional[List[Tuple[int, int, ConvW]]] = None
+
+
+def pack_transpose(w: torch.Tensor, bias: torch.Tensor, fmt: int, pack_sub: Callable[[int, int], torch.Tensor]) -> TransposeW:
+    """`w` [cin][cout][2][2] fp32; `pack_sub(a, b)`: the tensor-core storage of the K-major matrix w[:, :, a, b]^T."""
+    cin, cout = w.shape[0], w.shape[1]
+    if fmt == FMT_F32:
+        return TransposeW(bias, cin, cout, simt=w.permute(2, 3, 0, 1).reshape(4, cin, cout).contiguous())
+    return TransposeW(bias, cin, cout, subs=[(a, b, ConvW(pack_sub(a, b), bias, cin, cout, 1, 1)) for a in range(2) for b in range(2)])
+
+
+class InvStd(NamedTuple):
+    """Where the final layer reads 1/std: sample n of the current step takes values[n * stride + step * step_stride], with
+    step = *step_counter (0 without a counter); no values: no scaling.  A sampler passes its step table's 1/std column, stride 0,
+    the table's row length and the device step counter."""
+    values: Optional[torch.Tensor]
+    stride: int = 1
+    step_stride: int = 0
+    step_counter: Optional[torch.Tensor] = None
+
+    def args(self) -> tuple:
+        return _ptr(self.values), self.stride, self.step_stride, _ptr(self.step_counter)
 
 
 def _split_bf16(x: torch.Tensor) -> torch.Tensor:
@@ -165,6 +201,10 @@ class _Packer:
             km = w.permute(0, 2, 3, 1).reshape(cout, kh * kw * cin).contiguous()           # [cout][K]
             packed = pack_tc_matrix(km, self.fmt)
         return ConvW(packed, None if bias is None else bias.contiguous(), cin, cout, kh, kw)
+
+    def conv_transpose(self, wkey: str, bias_key: str) -> TransposeW:
+        w = self.get(wkey)                                    # [cin, cout, 2, 2]
+        return pack_transpose(w, self.vec(bias_key), self.fmt, lambda a, b: pack_tc_matrix(w[:, :, a, b].t().contiguous(), self.fmt))
 
 
 def _unpack_tc_matrix(packed: torch.Tensor, fmt: int) -> torch.Tensor:
@@ -316,7 +356,7 @@ class Kernels:
 
     def up_fused_ok(self, x: Act, cw: ConvW) -> bool:
         """True if conv3x3(upsample2x(x)) runs as ONE kernel (sbgm_conv3x3_c64_up): a 64 -> 64 convolution in a single-plane format."""
-        return (_UP_FUSED and self.fmt in (FMT_BF16, FMT_F16) and x.c == 64 and cw.cin == 64 and cw.cout == 64 and cw.kh == 3
+        return (self.fmt in (FMT_BF16, FMT_F16) and x.c == 64 and cw.cin == 64 and cw.cout == 64 and cw.kh == 3
                 and cw.kw == 3 and (2 * x.h) % 16 == 0 and (2 * x.w) % 8 == 0 and not _SKIP)
 
     def conv_up_fused(self, x: Act, cw: ConvW, proj: Optional[torch.Tensor] = None, gn_stats: bool = False):
@@ -343,15 +383,41 @@ class Kernels:
             return pout
         return (out, stats) if gn_stats else out
 
-    def affine(self, x: Act, skip: Optional[Act] = None, tproj: Optional[torch.Tensor] = None, act: int = ACT_NONE) -> Act:
-        """act(x + skip + tproj): the epilogue of a decoder block whose norm is nn.Identity (score_unet.py:593-612), as the
-        normalisation kernel with unit statistics (mean 0, rstd 1, no affine)."""
+    def affine(self, x: Act, skip: Optional[Act] = None, tproj: Optional[torch.Tensor] = None, act: int = ACT_NONE,
+               bias: Optional[torch.Tensor] = None) -> Act:
+        """act(x + bias + skip + tproj) as the normalisation kernel with unit statistics (mean 0, rstd 1, no gamma): the epilogue
+        of a decoder block whose norm is nn.Identity (score_unet.py:593-612), or the bias of the fp32 transposed convolution.
+        The tproj-before-activation flag is inert without a tproj; the bias form passes 0."""
         unit = torch.tensor([0.0, 1.0], dtype=torch.float32, device=self.device).repeat(x.c, 1).contiguous()
         out = x.like()
-        call("sbgm_norm_apply", x.ptr, x.plane, unit.data_ptr(), 2, x.c, None, None, None if skip is None else skip.ptr,
-             0 if skip is None else skip.plane, _ptr(tproj), tproj.stride(0) if tproj is not None else 0, 1, act, out.ptr, out.plane,
-             self.fmt, x.n, x.h * x.w, x.c, _stream())
+        call("sbgm_norm_apply", x.ptr, x.plane, unit.data_ptr(), 2, x.c, None, _ptr(bias), None if skip is None else skip.ptr,
+             0 if skip is None else skip.plane, _ptr(tproj), tproj.stride(0) if tproj is not None else 0, int(bias is None), act,
+             out.ptr, out.plane, self.fmt, x.n, x.h * x.w, x.c, _stream())
         return out
+
+    def conv_transpose2x(self, x: Act, tw: TransposeW) -> Act:
+        if self.fmt == FMT_F32:
+            # the data gradient of a (2x2, stride 2) convolution IS the transposed convolution; the bias is added afterwards
+            raw = Act(self.fmt, x.n, 2 * x.h, 2 * x.w, tw.cout, self.device)
+            call("sbgm_conv2d_dgrad_simt", x.ptr, x.plane, tw.simt.data_ptr(), raw.ptr, raw.plane, 0, self.fmt,
+                 x.n, 2 * x.h, 2 * x.w, tw.cout, tw.cin, 2, 2, 2, 0, _stream())
+            return self.affine(raw, bias=tw.bias)
+        out = Act(self.fmt, x.n, 2 * x.h, 2 * x.w, tw.cout, self.device)
+        for a, b, cw in tw.subs:
+            call("sbgm_conv2d_tc_ex", x.ptr, x.plane, cw.w.data_ptr(), cw.plane, cw.bias.data_ptr(), None, 0, 0, None, 0, out.ptr, out.plane,
+                 self.fmt, x.n, x.h, x.w, cw.cin, cw.cout, 1, 1, 1, 0, 0, x.h, x.w, 2 * x.h, 2 * x.w, 2, a, b, ACT_NONE, None, 0, _stream())
+        return out
+
+    def final_conv(self, a: Act, w: torch.Tensor, bias: torch.Tensor, inv_std: InvStd, out: torch.Tensor) -> None:
+        """out [n, cout, h, w] fp32 = (conv3x3(a, w) + bias) * 1/std: the decoder's final layer (`w` [cout][9][cin] fp32)."""
+        call("sbgm_final_conv", a.ptr, a.plane, self.fmt, w.data_ptr(), bias.data_ptr(), *inv_std.args(), out.data_ptr(),
+             a.n, a.h, a.w, a.c, w.shape[0], _stream())
+
+    def final_gather(self, proj: torch.Tensor, bias: torch.Tensor, inv_std: InvStd, out: torch.Tensor) -> None:
+        """The final 64 -> 1 layer from the nine per-tap partial products `proj` [n, h, w, PROJ_STRIDE] that conv_up's epilogue
+        emitted: out [n, 1, h, w] = (sum of the taps + bias) * 1/std."""
+        n, h, w = proj.shape[:3]
+        call("sbgm_final_gather", proj.data_ptr(), bias.data_ptr(), *inv_std.args(), out.data_ptr(), n, h, w, _stream())
 
     def layernorm(self, x: Act, gamma, beta) -> Act:
         if "ln" in _SKIP:
@@ -423,10 +489,7 @@ def attention_block(k: Kernels, aw: AttentionW, x: Act) -> Act:
         att = k.attention_core(qkv, b, s, c, aw.heads)
         h = k.linear(att, aw.out_proj, residual=tok)
     g = k.linear_ln(h, aw.ff0_ln, act=ACT_GELU) if fold else k.linear(k.layernorm(h, *aw.ln2), aw.ff0, act=ACT_GELU)
-    y = k.linear(g, aw.ff2, residual=h)
-    out = Act.__new__(Act)
-    out.buf, out.fmt, out.n, out.h, out.w, out.c = y.buf, y.fmt, x.n, x.h, x.w, x.c
-    return out
+    return k.linear(g, aw.ff2, residual=h).view(x.n, x.h, x.w, x.c)
 
 
 class TimeProjector:
@@ -606,7 +669,8 @@ class DecoderEngine:
             bp = f"{prefix}residual_layers.{i}"
             affine = norm == "group"
             blk = dict(
-                conv_up=pk.conv(f"{bp}.conv_up.weight", f"{bp}.conv_up.bias") if use_resize_conv else self._pack_transpose(pk, f"{bp}.transpose"),
+                conv_up=(pk.conv(f"{bp}.conv_up.weight", f"{bp}.conv_up.bias") if use_resize_conv else
+                         pk.conv_transpose(f"{bp}.transpose.weight", f"{bp}.transpose.bias")),
                 conv=pk.conv(f"{bp}.conv.weight", f"{bp}.conv.bias"),
                 n1=(pk.vec(f"{bp}.norm1.weight"), pk.vec(f"{bp}.norm1.bias")) if affine else (None, None),
                 n2=(pk.vec(f"{bp}.norm2.weight"), pk.vec(f"{bp}.norm2.bias")) if affine else (None, None),
@@ -618,49 +682,15 @@ class DecoderEngine:
             tp.add_head(f"dec{i}", s, pk.get(f"{bp}.time_projection_layer.1.weight"), pk.vec(f"{bp}.time_projection_layer.1.bias"))
             self.blocks.append(blk)
         fp = f"{prefix}final_layer"
-        self.final_up = pk.conv(f"{fp}.conv_up.weight", f"{fp}.conv_up.bias") if use_resize_conv else self._pack_transpose(pk, f"{fp}.transpose")
+        self.final_up = (pk.conv(f"{fp}.conv_up.weight", f"{fp}.conv_up.bias") if use_resize_conv else
+                         pk.conv_transpose(f"{fp}.transpose.weight", f"{fp}.transpose.bias"))
         wf = pk.get(f"{fp}.conv.weight")                                   # [cout, cin, 3, 3]
         self.final_w = wf.permute(0, 2, 3, 1).reshape(wf.shape[0], 9, wf.shape[1]).contiguous()
         self.final_b = pk.vec(f"{fp}.conv.bias")
         self.out_channels = out_channels
         self.tp = tp
 
-    def _pack_transpose(self, pk: _Packer, prefix: str):
-        """nn.ConvTranspose2d(c, c, kernel 2, stride 2) (score_unet.py:466-468, the use_resize_conv=False ablation):
-        out[n, 2i+a, 2j+b, co] = bias[co] + sum_ci x[n, i, j, ci] W[ci][co][a][b] -- four 1x1 convolutions scattered to
-        the four output parities (tensor cores), or one gather over the 2x2 taps (fp32 / CUDA cores)."""
-        w = pk.get(f"{prefix}.weight")                        # [cin, cout, 2, 2]
-        bias = pk.vec(f"{prefix}.bias")
-        cin, cout = w.shape[0], w.shape[1]
-        if self.fmt == FMT_F32:
-            return dict(simt=w.permute(2, 3, 0, 1).reshape(4, cin, cout).contiguous(), bias=bias, cin=cin, cout=cout)
-        subs = []
-        for a in range(2):
-            for b in range(2):
-                km = w[:, :, a, b].t().contiguous()          # [cout][cin] K-major
-                subs.append((a, b, ConvW(pack_tc_matrix(km, self.fmt), bias, cin, cout, 1, 1)))
-        return dict(subs=subs, bias=bias, cin=cin, cout=cout)
-
-    def _transpose_up(self, x: Act, tw: dict):
-        k = self.k
-        out = Act(self.fmt, x.n, 2 * x.h, 2 * x.w, tw["cout"], self.device)
-        if self.fmt == FMT_F32:
-            # the data gradient of a (2x2, stride 2) convolution IS the transposed convolution; bias via a unit-statistics affine
-            raw = Act(self.fmt, x.n, 2 * x.h, 2 * x.w, tw["cout"], self.device)
-            call("sbgm_conv2d_dgrad_simt", x.ptr, x.plane, tw["simt"].data_ptr(), raw.ptr, raw.plane, 0, self.fmt,
-                 x.n, 2 * x.h, 2 * x.w, tw["cout"], tw["cin"], 2, 2, 2, 0, _stream())
-            unit = torch.tensor([0.0, 1.0], dtype=torch.float32, device=self.device).repeat(tw["cout"], 1).contiguous()
-            call("sbgm_norm_apply", raw.ptr, raw.plane, unit.data_ptr(), 2, tw["cout"], None, tw["bias"].data_ptr(), None, 0, None, 0, 0,
-                 ACT_NONE, out.ptr, out.plane, self.fmt, x.n, 4 * x.h * x.w, tw["cout"], _stream())
-            return out
-        for a, b, cw in tw["subs"]:
-            call("sbgm_conv2d_tc_ex", x.ptr, x.plane, cw.w.data_ptr(), cw.plane, cw.bias.data_ptr(), None, 0, 0, None, 0, out.ptr, out.plane,
-                 self.fmt, x.n, x.h, x.w, cw.cin, cw.cout, 1, 1, 1, 0, 0, x.h, x.w, 2 * x.h, 2 * x.w, 2, a, b, ACT_NONE, None, 0, _stream())
-        return out
-
-    def forward(self, fmaps: List[Act], tproj: torch.Tensor, inv_std: Optional[torch.Tensor], *,
-                inv_std_stride: int = 1, inv_std_step_stride: int = 0, step_counter: Optional[torch.Tensor] = None,
-                dst: Optional[torch.Tensor] = None) -> torch.Tensor:
+    def forward(self, fmaps: List[Act], tproj: torch.Tensor, inv_std: InvStd, dst: Optional[torch.Tensor] = None) -> torch.Tensor:
         k, tp = self.k, self.tp
         rev = list(reversed(fmaps))
         out = rev[0]
@@ -671,7 +701,7 @@ class DecoderEngine:
                 up = k.upsample2x(out)
                 a, st1 = k.conv(up, blk["conv_up"], pad=1, gn_stats=True)
             else:
-                a, st1 = self._transpose_up(out, blk["conv_up"]), None
+                a, st1 = k.conv_transpose2x(out, blk["conv_up"]), None
             a = k.groupnorm(a, *blk["n1"], groups=blk["g1"], stats=st1)
             b, st2 = k.conv(a, blk["conv"], pad=1, gn_stats=True)
             skip = rev[i + 1]
@@ -681,40 +711,26 @@ class DecoderEngine:
                               stats=st2)
             if blk["attn"] is not None:
                 out = attention_block(k, blk["attn"], out)
-        if self.use_resize_conv and isinstance(self.final_up, ConvW) and k.up_fused_ok(out, self.final_up):
-            n, h, w = out.n, 2 * out.h, 2 * out.w
-            res = dst if dst is not None else torch.empty((n, self.out_channels, h, w), dtype=torch.float32, device=self.device)
+        # the final layer: conv_up's output `a` for the final convolution, or the final 64 -> 1 convolution's per-tap partial
+        # products `pr` out of conv_up's epilogue (its 64-channel output never reaches HBM; tc_common.cuh: projection epilogue)
+        a = pr = None
+        if self.use_resize_conv and k.up_fused_ok(out, self.final_up):
             if self.out_channels == 1:
                 pr = k.conv_up_fused(out, self.final_up, proj=self.final_w[0])
-                call("sbgm_final_gather", pr.data_ptr(), self.final_b.data_ptr(), _ptr(inv_std), inv_std_stride,
-                     inv_std_step_stride, _ptr(step_counter), res.data_ptr(), n, h, w, _stream())
-                return res
-            a = k.conv_up_fused(out, self.final_up)
-            call("sbgm_final_conv", a.ptr, a.plane, self.fmt, self.final_w.data_ptr(), self.final_b.data_ptr(), _ptr(inv_std),
-                 inv_std_stride, inv_std_step_stride, _ptr(step_counter), res.data_ptr(), a.n, a.h, a.w, a.c,
-                 self.out_channels, _stream())
-            return res
-        if not self.use_resize_conv:
-            a = self._transpose_up(out, self.final_up)
-            res = dst if dst is not None else torch.empty((a.n, self.out_channels, a.h, a.w), dtype=torch.float32, device=self.device)
-            call("sbgm_final_conv", a.ptr, a.plane, self.fmt, self.final_w.data_ptr(), self.final_b.data_ptr(), _ptr(inv_std),
-                 inv_std_stride, inv_std_step_stride, _ptr(step_counter), res.data_ptr(), a.n, a.h, a.w, a.c,
-                 self.out_channels, _stream())
-            return res
-        up = k.upsample2x(out)
-        n, h, w = up.n, up.h, up.w
+            else:
+                a = k.conv_up_fused(out, self.final_up)
+        elif not self.use_resize_conv:
+            a = k.conv_transpose2x(out, self.final_up)
+        elif self.fmt != FMT_F32 and self.out_channels == 1 and self.final_up.cout == 64:
+            pr = k.conv(k.upsample2x(out), self.final_up, pad=1, proj=self.final_w[0])
+        else:
+            a = k.conv(k.upsample2x(out), self.final_up, pad=1)
+        n, h, w = (a.n, a.h, a.w) if pr is None else pr.shape[:3]
         res = dst if dst is not None else torch.empty((n, self.out_channels, h, w), dtype=torch.float32, device=self.device)
-        if self.fmt != FMT_F32 and self.out_channels == 1 and self.final_up.cout == 64:
-            # conv_up's epilogue emits the 9 per-tap partial products of the final 64->1 convolution; its
-            # 64-channel output never reaches HBM (tc_common.cuh: projection epilogue)
-            pr = k.conv(up, self.final_up, pad=1, proj=self.final_w[0])
-            call("sbgm_final_gather", pr.data_ptr(), self.final_b.data_ptr(), _ptr(inv_std), inv_std_stride,
-                 inv_std_step_stride, _ptr(step_counter), res.data_ptr(), n, h, w, _stream())
-            return res
-        a = k.conv(up, self.final_up, pad=1)
-        call("sbgm_final_conv", a.ptr, a.plane, self.fmt, self.final_w.data_ptr(), self.final_b.data_ptr(), _ptr(inv_std),
-             inv_std_stride, inv_std_step_stride, _ptr(step_counter), res.data_ptr(), a.n, a.h, a.w, a.c,
-             self.out_channels, _stream())
+        if pr is None:
+            k.final_conv(a, self.final_w, self.final_b, inv_std, res)
+        else:
+            k.final_gather(pr, self.final_b, inv_std, res)
         return res
 
 
@@ -748,16 +764,22 @@ class UNetSpec:
     activation: str = "silu"
 
 
+def engine_device(precision: str, device) -> torch.device:
+    """Check an engine's precision name and device and load the library; returns the device."""
+    if precision not in PRECISIONS:
+        raise ValueError(f"precision must be one of {sorted(PRECISIONS)}, got {precision!r}")
+    device = torch.device(device)
+    if device.type != "cuda":
+        raise RuntimeError("sbgm_danra_b200 runs on CUDA devices only (no CPU fallback); got device " + str(device))
+    _lib.load_library()
+    return device
+
+
 class UNetEngine:
     """Encoder + decoder + time projector packed for one (state-dict, precision, device)."""
 
     def __init__(self, sd: Dict[str, torch.Tensor], spec: UNetSpec, precision: str, device) -> None:
-        if precision not in PRECISIONS:
-            raise ValueError(f"precision must be one of {sorted(PRECISIONS)}, got {precision!r}")
-        device = torch.device(device)
-        if device.type != "cuda":
-            raise RuntimeError("sbgm_danra_b200 runs on CUDA devices only (no CPU fallback); got device " + str(device))
-        _lib.load_library()
+        device = engine_device(precision, device)
         self.spec, self.precision, self.device = spec, precision, device
         self.fmt = PRECISIONS[precision]
         with torch.cuda.device(device), torch.no_grad():
@@ -784,4 +806,4 @@ class UNetEngine:
             x = x.to(device=self.device, dtype=torch.float32).contiguous()
             tproj = self.tp(t, y)
             fmaps = self.enc.forward(x, planes, tproj)
-            return self.dec.forward(fmaps, tproj, inv_std)
+            return self.dec.forward(fmaps, tproj, InvStd(inv_std))

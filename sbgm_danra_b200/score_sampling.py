@@ -161,8 +161,8 @@ class _NativeStep:
         self.eng, self.dev, self.b, self.size = eng, eng.device, batch, size
         dev = self.dev
         self.table = torch.zeros((n_steps, STEP_COLS), dtype=torch.float32, device=dev)
-        self.inv_std = self.table[:, 3]
         self.counter = torch.zeros(4, dtype=torch.int32, device=dev)       # step, scratch, seed lo, seed hi
+        self.inv_std = _eng.InvStd(self.table[:, 3], 0, STEP_COLS, self.counter)
         self.x = torch.zeros((batch, 1, size, size), dtype=torch.float32, device=dev)
         self.score = torch.empty_like(self.x)
         self.mean = torch.empty_like(self.x)
@@ -223,10 +223,7 @@ class _NativeStep:
             self.eng.tp(self.table, None, rows=self.table.shape[0], t_row_stride=STEP_COLS, t_step_stride=0, out=self.tproj_all)
         if self.y is not None:
             self.y.copy_(y.to(device=self.dev, dtype=torch.int64).reshape(-1))
-        if self.partial is not None:
-            self.eng.enc.stem_partial(planes, self.size, self.size, out=self.partial)
-            if self.cfg_scale is not None:
-                self.eng.enc.stem_partial(planes_u, self.size, self.size, out=self.partial_u)
+        self._load_planes(planes, planes_u)
         if self.wide:
             if self.y2 is not None:
                 self.y2[:self.b].copy_(self.y)
@@ -240,20 +237,26 @@ class _NativeStep:
                     shape = tuple(dst_t.shape[:nd]) + (self.b,) + tuple(dst_t.shape[nd + 1:])
                     dst_t[dsl].copy_(src_t.expand(shape) if src_t.shape[nd] == 1 else src_t)
 
+    def _load_planes(self, planes, planes_u) -> None:
+        """The stem's step-invariant contribution of the conditioning planes (and of the null branch's)."""
+        if self.partial is not None:
+            self.eng.enc.stem_partial(planes, self.size, self.size, out=self.partial)
+            if self.cfg_scale is not None:
+                self.eng.enc.stem_partial(planes_u, self.size, self.size, out=self.partial_u)
+
     def _forward(self, partial, y, tproj, out, x=None) -> None:
-        eng = self.eng
         x = self.x if x is None else x
         if self.tproj_all is not None:
             call("sbgm_select_step_row", self.tproj_all.data_ptr(), self.tproj_all.shape[1], self.counter.data_ptr(),
                  self.tproj_row.data_ptr(), _eng._stream())
         else:
-            eng.tp(self.table, y, rows=x.shape[0], t_row_stride=0, t_step_stride=STEP_COLS, step_counter=self.counter, out=tproj)
-        if partial is None:
-            fmaps = eng.enc.forward(x, None, tproj)
-        else:
-            fmaps = eng.enc.forward(x, None, tproj, partial=partial)
-        eng.dec.forward(fmaps, tproj, self.inv_std, inv_std_stride=0, inv_std_step_stride=STEP_COLS,
-                        step_counter=self.counter, dst=out)
+            self.eng.tp(self.table, y, rows=x.shape[0], t_row_stride=0, t_step_stride=STEP_COLS, step_counter=self.counter, out=tproj)
+        self._evaluate(x, partial, y, tproj, out)
+
+    def _evaluate(self, x, partial, y, tproj, out) -> None:
+        """The network at the step's time projections `tproj` into `out`; `partial`: the conditioning as `_load_planes` left it."""
+        fmaps = self.eng.enc.forward(x, None, tproj, partial=partial)
+        self.eng.dec.forward(fmaps, tproj, self.inv_std, dst=out)
 
     def score_into(self, scale: Optional[float] = None) -> torch.Tensor:
         """`scale`: guidance scale of THIS evaluation (the PC corrector clamps it to guidance_scale_max, the predictor does
@@ -298,29 +301,16 @@ class _TrainModeStep(_NativeStep):
         self.partial = None if planes is None else torch.empty_like(planes)
         self.partial_u = None if planes_u is None else torch.empty_like(planes_u)
 
-    def load(self, table: torch.Tensor, seed: int, y, planes, planes_u) -> None:
-        self.table.copy_(table)
-        self.counter.copy_(torch.tensor(_seed_words(seed), dtype=torch.int32))
-        if self.tproj_all is not None:
-            self.eng.tp(self.table, None, rows=self.table.shape[0], t_row_stride=STEP_COLS, t_step_stride=0, out=self.tproj_all)
-        if self.y is not None:
-            self.y.copy_(y.to(device=self.dev, dtype=torch.int64).reshape(-1))
+    def _load_planes(self, planes, planes_u) -> None:
         if self.partial is not None:
             self.partial.copy_(planes)
         if self.partial_u is not None:
             self.partial_u.copy_(planes_u)
 
-    def _forward(self, partial, y, tproj, out, x=None) -> None:
-        x = self.x if x is None else x
-        if self.tproj_all is not None:
-            call("sbgm_select_step_row", self.tproj_all.data_ptr(), self.tproj_all.shape[1], self.counter.data_ptr(),
-                 self.tproj_row.data_ptr(), _eng._stream())
-        else:
-            self.eng.tp(self.table, y, rows=x.shape[0], t_row_stride=0, t_step_stride=STEP_COLS, step_counter=self.counter, out=tproj)
+    def _evaluate(self, x, partial, y, tproj, out) -> None:
         # weights were packed when the plan was built (the plan is keyed on the parameter versions); the running statistics are
         # read and updated live
-        self.train_eng.forward(x, None, y, partial, None,
-                               sampler=dict(tproj=tproj, inv_std=(self.inv_std, 0, STEP_COLS, self.counter), dst=out))
+        self.train_eng.forward(x, None, y, partial, None, sampler=dict(tproj=tproj, inv_std=self.inv_std, dst=out))
         torch._foreach_add_(self.bn_counters, 1)
 
 

@@ -311,7 +311,7 @@ class DecoderBlock(nn.Module):
                 else:                                   # a precomputed embedding [B, time_dim]: SiLU -> Linear on the kernels
                     tcols = self._project_embedding(k, t.float(), fmt)
             x = _eng.Act.from_nchw(fmap.to(dev), fmt)
-            a = k.conv(k.upsample2x(x), blk["conv_up"], pad=1) if self.use_resize_conv else de._transpose_up(x, blk["conv_up"])
+            a = k.conv(k.upsample2x(x), blk["conv_up"], pad=1) if self.use_resize_conv else k.conv_transpose2x(x, blk["conv_up"])
             if not id1:
                 a = k.groupnorm(a, *blk["n1"], groups=blk["g1"])
             b = k.conv(a, blk["conv"], pad=1)
@@ -399,7 +399,7 @@ class Decoder(nn.Module):
             dec, fmt = self._engine()
             acts = [_eng.Act.from_nchw(f.to(dev), fmt) for f in fmaps]
             tproj = dec.tp(t.to(dev), None)
-            return dec.forward(acts, tproj, None)
+            return dec.forward(acts, tproj, _eng.InvStd(None))
 
 
 class ScoreNet(nn.Module):

@@ -21,7 +21,8 @@ import torch
 from . import _lib
 from ._capture import graph_capture
 from ._lib import ACT_GELU, ACT_NONE, ACT_RELU, FMT_BF16X2, FMT_F32, call
-from .engine import ACTS, BN_EPS, GN_EPS, LN_EPS, PRECISIONS, Act, ConvW, Kernels, UNetSpec, _ptr, _stream
+from .engine import (ACTS, BN_EPS, GN_EPS, LN_EPS, PRECISIONS, Act, ConvW, InvStd, Kernels, UNetSpec, _ptr, _stream, engine_device,
+                     pack_transpose)
 
 BN_MOMENTUM = 0.1
 # "fp16x2" is an inference storage format (engine.py); a model set to it trains on the bf16x3 kernels
@@ -156,13 +157,8 @@ class ConvTLayer:
         self.name, self.bias_name, self.fmt = name, bias_name, fmt
         self.w, self.shape = w.contiguous(), tuple(w.shape)
         self.cin, self.cout = w.shape[0], w.shape[1]
-        self.bias = bias.contiguous()
         self.back = ConvW(_pack_oihw(self.w, fmt), None, self.cout, self.cin, 2, 2)          # C: cout channels in, cin out
-        if fmt == FMT_F32:
-            self.fwd_simt = self.w.permute(2, 3, 0, 1).reshape(4, self.cin, self.cout).contiguous()
-        else:
-            self.fwd_subs = [(a, b, ConvW(_pack_tc(self.w, fmt, [a * 2 + b], True), self.bias, self.cin, self.cout, 1, 1))
-                             for a in range(2) for b in range(2)]
+        self.fwd = pack_transpose(self.w, bias.contiguous(), fmt, lambda a, b: _pack_tc(self.w, fmt, [a * 2 + b], True))
 
 
 class Tape:
@@ -184,9 +180,7 @@ class Tape:
         if g is not None and (g.n, g.h, g.w, g.c) != (a.n, a.h, a.w, a.c):
             # the gradient was deposited through a view (tokens <-> image): same storage, the consumer's geometry
             assert g.plane == a.plane
-            v = Act.__new__(Act)
-            v.buf, v.fmt, v.n, v.h, v.w, v.c = g.buf, g.fmt, a.n, a.h, a.w, a.c
-            return v
+            return g.view(a.n, a.h, a.w, a.c)
         return g
 
     def add(self, a: Act, g: Act) -> None:
@@ -224,6 +218,25 @@ class TrainKernels:
             self._scratch[tag] = cur
         return cur
 
+    def channel_sums(self, dy: Act, dtproj: Optional[torch.Tensor] = None, dbias: Optional[torch.Tensor] = None) -> None:
+        """dy summed over the pixels into the rows of `dtproj` (per sample) and / or over the batch too into `dbias`."""
+        ws = self.scratch("chansum", _lib.query("sbgm_channel_sums_scratch_floats", dy.n, dy.c), tickets=True)
+        call("sbgm_channel_sums", dy.ptr, dy.plane, self.fmt, dy.n, dy.h * dy.w, dy.c, _ptr(dtproj), 0 if dtproj is None else dtproj.stride(0),
+             _ptr(dbias), ws.data_ptr(), _stream())
+
+    def wgrad(self, x: Act, dy: Act, dw: torch.Tensor, cin: int, cout: int, kh: int, kw: int, stride: int, pad: int) -> bool:
+        """dw [cout][cin][kh][kw] of the convolution x -> dy, on the tensor cores where both channel counts are multiples of 64,
+        else on the CUDA cores.  Returns True for the tensor cores."""
+        fmt, args = self.fmt, (x.n, x.h, x.w, cin, cout, kh, kw, stride, pad)
+        tc = fmt != FMT_F32 and cin % 64 == 0 and cout % 64 == 0
+        if tc:
+            ws = self.scratch("wgrad", _lib.query("sbgm_conv2d_wgrad_tc_workspace_floats", fmt, *args))
+            call("sbgm_conv2d_wgrad_tc", x.ptr, x.plane, dy.ptr, dy.plane, dw.data_ptr(), fmt, *args, ws.data_ptr(), _stream())
+        else:
+            ws = self.scratch("wgrad", _lib.query("sbgm_conv2d_wgrad_simt_workspace_floats", *args))
+            call("sbgm_conv2d_wgrad_simt", x.ptr, x.plane, dy.ptr, dy.plane, dw.data_ptr(), fmt, *args, ws.data_ptr(), _stream())
+        return tc
+
     def grad_like(self, a: Act, zero: bool = False) -> Act:
         g = Act(self.fmt, a.n, a.h, a.w, a.c, self.device)
         if zero:
@@ -256,9 +269,7 @@ class TrainKernels:
             if residual is not None:
                 tape.add(residual, dy)
             if dtproj is not None:
-                ws = self.scratch("chansum", _lib.query("sbgm_channel_sums_scratch_floats", dy.n, dy.c), tickets=True)
-                call("sbgm_channel_sums", dy.ptr, dy.plane, self.fmt, dy.n, dy.h * dy.w, dy.c, dtproj.data_ptr(), dtproj.stride(0), None,
-                     ws.data_ptr(), _stream())
+                self.channel_sums(dy, dtproj=dtproj)
 
         tape.record(backward, x, y)
         if proj is not None:
@@ -270,20 +281,8 @@ class TrainKernels:
         n, h, w = x.n, x.h, x.w
         cin, cout, kh, kw = layer.cin, layer.cout, layer.kh, layer.kw
         if layer.bias_name is not None and bias_grad:
-            db = self.param_grad(layer.bias_name, (cout,))
-            ws = self.scratch("chansum", _lib.query("sbgm_channel_sums_scratch_floats", dy.n, cout), tickets=True)
-            call("sbgm_channel_sums", dy.ptr, dy.plane, fmt, dy.n, dy.h * dy.w, cout, None, 0, db.data_ptr(), ws.data_ptr(), st)
-        tc = fmt != FMT_F32 and cin % 64 == 0 and cout % 64 == 0
-        if tc:
-            dw = self.param_grad(layer.name, layer.shape)
-            ws = self.scratch("wgrad", _lib.query("sbgm_conv2d_wgrad_tc_workspace_floats", fmt, n, h, w, cin, cout, kh, kw, stride, pad))
-            call("sbgm_conv2d_wgrad_tc", x.ptr, x.plane, dy.ptr, dy.plane, dw.data_ptr(), fmt, n, h, w, cin, cout, kh, kw, stride, pad,
-                 ws.data_ptr(), st)
-        else:
-            dw = self.param_grad(layer.name, layer.shape)
-            ws = self.scratch("wgrad", _lib.query("sbgm_conv2d_wgrad_simt_workspace_floats", n, h, w, cin, cout, kh, kw, stride, pad))
-            call("sbgm_conv2d_wgrad_simt", x.ptr, x.plane, dy.ptr, dy.plane, dw.data_ptr(), fmt, n, h, w, cin, cout, kh, kw, stride, pad,
-                 ws.data_ptr(), st)
+            self.channel_sums(dy, dbias=self.param_grad(layer.bias_name, (cout,)))
+        tc = self.wgrad(x, dy, self.param_grad(layer.name, layer.shape), cin, cout, kh, kw, stride, pad)
         if not need_dx:
             return
         tape = self.tape
@@ -451,37 +450,16 @@ class TrainKernels:
         return y
 
     def conv_transpose2x(self, x: Act, layer: ConvTLayer) -> Act:
-        fmt, st = self.fmt, _stream()
-        y = Act(fmt, x.n, 2 * x.h, 2 * x.w, layer.cout, self.device)
-        if fmt == FMT_F32:
-            raw = Act(fmt, x.n, 2 * x.h, 2 * x.w, layer.cout, self.device)
-            call("sbgm_conv2d_dgrad_simt", x.ptr, x.plane, layer.fwd_simt.data_ptr(), raw.ptr, raw.plane, 0, fmt,
-                 x.n, 2 * x.h, 2 * x.w, layer.cout, layer.cin, 2, 2, 2, 0, st)
-            unit = torch.tensor([0.0, 1.0], dtype=torch.float32, device=self.device).repeat(layer.cout, 1).contiguous()
-            call("sbgm_norm_apply", raw.ptr, raw.plane, unit.data_ptr(), 2, layer.cout, None, layer.bias.data_ptr(), None, 0, None, 0, 0,
-                 ACT_NONE, y.ptr, y.plane, fmt, x.n, 4 * x.h * x.w, layer.cout, st)
-        else:
-            for a, b, cw in layer.fwd_subs:
-                call("sbgm_conv2d_tc_ex", x.ptr, x.plane, cw.w.data_ptr(), cw.plane, cw.bias.data_ptr(), None, 0, 0, None, 0, y.ptr, y.plane,
-                     fmt, x.n, x.h, x.w, cw.cin, cw.cout, 1, 1, 1, 0, 0, x.h, x.w, 2 * x.h, 2 * x.w, 2, a, b, ACT_NONE, None, 0, st)
+        y = self.k.conv_transpose2x(x, layer.fwd)
         tape = self.tape
 
         def backward() -> None:
             dy = tape.pop(y)
             if dy is None:
                 return
-            s2 = _stream()
-            db = self.param_grad(layer.bias_name, (layer.cout,))
-            ws = self.scratch("chansum", _lib.query("sbgm_channel_sums_scratch_floats", dy.n, layer.cout), tickets=True)
-            call("sbgm_channel_sums", dy.ptr, dy.plane, fmt, dy.n, dy.h * dy.w, layer.cout, None, 0, db.data_ptr(), ws.data_ptr(), s2)
-            dw = self.param_grad(layer.name, layer.shape)
-            args = (dy.n, dy.h, dy.w, layer.cout, layer.cin, 2, 2, 2, 0)      # C: input dy-grid (cout channels), output x-grid
-            if fmt != FMT_F32 and layer.cin % 64 == 0 and layer.cout % 64 == 0:
-                wsw = self.scratch("wgrad", _lib.query("sbgm_conv2d_wgrad_tc_workspace_floats", fmt, *args))
-                call("sbgm_conv2d_wgrad_tc", dy.ptr, dy.plane, x.ptr, x.plane, dw.data_ptr(), fmt, *args, wsw.data_ptr(), s2)
-            else:
-                wsw = self.scratch("wgrad", _lib.query("sbgm_conv2d_wgrad_simt_workspace_floats", *args))
-                call("sbgm_conv2d_wgrad_simt", dy.ptr, dy.plane, x.ptr, x.plane, dw.data_ptr(), fmt, *args, wsw.data_ptr(), s2)
+            self.channel_sums(dy, dbias=self.param_grad(layer.bias_name, (layer.cout,)))
+            # C: input dy-grid (cout channels), output x-grid
+            self.wgrad(dy, x, self.param_grad(layer.name, layer.shape), layer.cout, layer.cin, 2, 2, 2, 0)
             tape.add(x, self.k.conv(dy, layer.back, stride=2, pad=0))
 
         tape.record(backward, x, y)
@@ -545,10 +523,7 @@ def _attention_block(tk: TrainKernels, aw: _AttnLayers, x: Act) -> Act:
     g = tk.layernorm(h, *aw.ln2, f"{p}.ln2.weight", f"{p}.ln2.bias")
     g1 = tk.conv(g, aw.ff0)
     g2 = tk.activation(g1, ACT_GELU)
-    y = tk.conv(g2, aw.ff2, residual=h)
-    out = Act.__new__(Act)
-    out.buf, out.fmt, out.n, out.h, out.w, out.c = y.buf, y.fmt, x.n, x.h, x.w, x.c
-    return out
+    return tk.conv(g2, aw.ff2, residual=h).view(x.n, x.h, x.w, x.c)
 
 
 class TrainEngine:
@@ -561,12 +536,7 @@ class TrainEngine:
                  encoder_only: bool = False) -> None:
         """`encoder_only`: `params` holds the encoder alone and `forward` returns its five feature maps (the standalone
         `Encoder.forward` in .train(): batch statistics, running statistics updated; nothing is differentiated)."""
-        if precision not in PRECISIONS:
-            raise ValueError(f"precision must be one of {sorted(PRECISIONS)}, got {precision!r}")
-        device = torch.device(device)
-        if device.type != "cuda":
-            raise RuntimeError("sbgm_danra_b200 runs on CUDA devices only (no CPU fallback); got device " + str(device))
-        _lib.load_library()
+        device = engine_device(precision, device)
         self.spec, self.device, self.fmt, self.bn_train = spec, device, TRAIN_PRECISIONS[precision], bn_train
         self.encoder_only = encoder_only
         self.sd = {k: v.detach() for k, v in params.items()}
@@ -680,8 +650,8 @@ class TrainEngine:
     def forward(self, x: torch.Tensor, t: Optional[torch.Tensor], y: Optional[torch.Tensor], planes: Optional[torch.Tensor],
                 inv_std: Optional[torch.Tensor], *, sampler: Optional[dict] = None) -> torch.Tensor:
         """`sampler` (score_sampling._TrainModeStep: a sampler step with batch-statistics BatchNorm, captured in a CUDA graph):
-        dict(tproj=[n, c_total] time projections already computed for the step, inv_std=(table column, row stride, step stride,
-        device step counter), dst=output tensor); no gradient buffer is set up and the recorded tape is dropped."""
+        dict(tproj=[n, c_total] time projections already computed for the step, inv_std=engine.InvStd of the step table's 1/std
+        column, dst=output tensor); no gradient buffer is set up and the recorded tape is dropped."""
         tk, fmt, dev = self.tk, self.fmt, self.device
         tape = Tape(fmt, dev)
         tk.tape = tape
@@ -720,9 +690,7 @@ class TrainEngine:
             df = tape.pop(f1)
             if df is None:
                 return
-            d0 = col(dtproj, "enc0")
-            ws = tk.scratch("chansum", _lib.query("sbgm_channel_sums_scratch_floats", n, 64), tickets=True)
-            call("sbgm_channel_sums", df.ptr, df.plane, fmt, n, f1.h * f1.w, 64, d0.data_ptr(), d0.stride(0), None, ws.data_ptr(), _stream())
+            tk.channel_sums(df, dtproj=col(dtproj, "enc0"))
             dw = self._param_grad("encoder.conv1.weight", (64, self.cin, 8, 8))
             ws2 = tk.scratch("stem", _lib.query("sbgm_stem_wgrad_workspace_floats", self.cin))
             call("sbgm_stem_wgrad", x.data_ptr(), _ptr(planes), 1 if planes is None else planes.shape[0], cc, df.ptr, df.plane, fmt,
@@ -775,22 +743,21 @@ class TrainEngine:
         smp = getattr(self, "_sampler", None)
         res = smp["dst"] if smp is not None else torch.empty((n, 1, 2 * out.h, 2 * out.w), dtype=torch.float32, device=dev)
         # 1 / std per member (training) or per sampler step (row of the step table selected by the device step counter)
-        iv = (_ptr(inv_std), 1, 0, None) if smp is None else (_ptr(smp["inv_std"][0]), smp["inv_std"][1], smp["inv_std"][2],
-                                                               _ptr(smp["inv_std"][3]))
-        up = tk.upsample2x(out) if self.spec.use_resize_conv else None
-        if up is None:
+        iv = InvStd(inv_std) if smp is None else smp["inv_std"]
+        pr = None
+        if not self.spec.use_resize_conv:
             a = tk.conv_transpose2x(out, self.final_up)
-            call("sbgm_final_conv", a.ptr, a.plane, fmt, self.final_w.data_ptr(), self.final_b.data_ptr(), *iv,
-                 res.data_ptr(), a.n, a.h, a.w, a.c, 1, _stream())
-        elif fmt != FMT_F32 and tk.k._c64_ok(up, self.final_up.fwd, 1, 1):
-            # the 64 -> 1 convolution rides in conv_up's epilogue (projection); conv_up's output is kept for the backward
-            a, pr = tk.conv(up, self.final_up, pad=1, proj=self.final_w[0], bias_grad=not self._final_bias_fused())
-            call("sbgm_final_gather", pr.data_ptr(), self.final_b.data_ptr(), *iv, res.data_ptr(), a.n, a.h, a.w,
-                 _stream())
         else:
-            a = tk.conv(up, self.final_up, pad=1, bias_grad=not self._final_bias_fused())
-            call("sbgm_final_conv", a.ptr, a.plane, fmt, self.final_w.data_ptr(), self.final_b.data_ptr(), *iv,
-                 res.data_ptr(), a.n, a.h, a.w, a.c, 1, _stream())
+            up = tk.upsample2x(out)
+            if fmt != FMT_F32 and tk.k._c64_ok(up, self.final_up.fwd, 1, 1):
+                # the 64 -> 1 convolution rides in conv_up's epilogue (projection); conv_up's output is kept for the backward
+                a, pr = tk.conv(up, self.final_up, pad=1, proj=self.final_w[0], bias_grad=not self._final_bias_fused())
+            else:
+                a = tk.conv(up, self.final_up, pad=1, bias_grad=not self._final_bias_fused())
+        if pr is None:
+            tk.k.final_conv(a, self.final_w, self.final_b, iv, res)
+        else:
+            tk.k.final_gather(pr, self.final_b, iv, res)
         if smp is not None:                    # a sampler step: nothing will run backward -- drop the tape and its activations
             self.tape = tk.tape = None
             self._final = self._time = self._sampler = None

@@ -357,6 +357,22 @@ def test_score_256x256_matches_oracle():
     assert rel_l2(got, want) < 1e-3
 
 
+@pytest.mark.parametrize("use_resize_conv", [True, False])
+@pytest.mark.parametrize("precision", ["fp32", "bf16x3", "fp16x2", "bf16"])
+def test_two_output_channels_match_oracle(precision, use_resize_conv):
+    """A final layer with two output channels (the reference trains with one): the final 3x3 convolution as its own kernel behind
+    every up-path -- the upsample inside conv_up (bf16 / fp16x2), the two-launch resize and the ConvTranspose2d."""
+    from oracle import score_ref
+    from oracle.synth import synth_batch
+    net, cfg, sd = _model(dict(n_lr=1, out_channels=2, use_resize_conv=use_resize_conv), precision)
+    b = synth_batch(batch=2, size=64, n_lr=1)
+    with torch.no_grad():
+        want = score_ref.score_forward(sd, cfg, *b.model_args())
+        got = net(*[_cuda(v) for v in b.model_args()]).cpu()
+    assert got.shape == want.shape == (2, 2, 64, 64)
+    assert rel_l2(got, want) < SCORE_TOL[precision]
+
+
 def test_non_power_of_two_size_matches_oracle():
     """96x96 input (feature maps 48/24/12/6/3): tiles with padding rows, odd attention lengths."""
     from oracle import score_ref
@@ -730,7 +746,7 @@ def test_upsample_inside_conv_up_is_bit_identical_to_the_two_launch_path(monkeyp
         fused = net(*args).clone()
     assert any(rec.get("up_fused") for rec in trace), "the fused path did not run"
     monkeypatch.setattr(E, "CONV_TRACE", None)
-    monkeypatch.setattr(E, "_UP_FUSED", False)
+    monkeypatch.setattr(E.Kernels, "up_fused_ok", lambda self, x, cw: False)
     with torch.no_grad():
         plain = net(*args).clone()
     assert torch.equal(fused, plain)

@@ -19,6 +19,7 @@ Precisions
 """
 from __future__ import annotations
 
+from collections import namedtuple
 from dataclasses import dataclass
 from typing import Callable, Dict, List, NamedTuple, Optional, Sequence, Tuple
 
@@ -184,15 +185,16 @@ class _Packer:
     def vec(self, key: str) -> torch.Tensor:
         return self.get(key).contiguous()
 
-    def conv(self, wkey: str, bias_key: Optional[str] = None, bn: Optional[str] = None) -> ConvW:
+    def conv(self, wkey: str, bias_key: Optional[str] = None, bn=None) -> ConvW:
         w = self.get(wkey)
         if w.dim() == 2:
             w = w[:, :, None, None]
         cout, cin, kh, kw = w.shape
         bias = self.get(bias_key) if bias_key is not None else None
         if bn is not None:   # eval-mode BatchNorm folded into the convolution
-            scale = self.get(f"{bn}.weight") / torch.sqrt(self.get(f"{bn}.running_var") + BN_EPS)
-            shift = self.get(f"{bn}.bias") - self.get(f"{bn}.running_mean") * scale
+            bn = batchnorm_keys(bn) if isinstance(bn, str) else bn      # the BatchNorm2d's key prefix or its BatchNormKeys
+            scale = self.get(bn.weight) / torch.sqrt(self.get(bn.running_var) + BN_EPS)
+            shift = self.get(bn.bias) - self.get(bn.running_mean) * scale
             w = w * scale[:, None, None, None]
             bias = shift if bias is None else bias * scale + shift
         if self.fmt == FMT_F32:
@@ -205,6 +207,9 @@ class _Packer:
     def conv_transpose(self, wkey: str, bias_key: str) -> TransposeW:
         w = self.get(wkey)                                    # [cin, cout, 2, 2]
         return pack_transpose(w, self.vec(bias_key), self.fmt, lambda a, b: pack_tc_matrix(w[:, :, a, b].t().contiguous(), self.fmt))
+
+    def up(self, site: "Affine", resize: bool):          # a decoder up-path: resize convolution (ConvW) or transposed one (TransposeW)
+        return self.conv(*site) if resize else self.conv_transpose(*site)
 
 
 def _unpack_tc_matrix(packed: torch.Tensor, fmt: int) -> torch.Tensor:
@@ -459,20 +464,19 @@ class Kernels:
 
 
 class AttentionW:
-    def __init__(self, pk: _Packer, prefix: str, heads: int) -> None:
+    def __init__(self, pk: _Packer, keys: "AttnKeys", heads: int) -> None:
         self.heads = heads
-        self.ln1 = (pk.vec(f"{prefix}.ln1.weight"), pk.vec(f"{prefix}.ln1.bias"))
-        self.ln2 = (pk.vec(f"{prefix}.ln2.weight"), pk.vec(f"{prefix}.ln2.bias"))
-        self.in_proj = pk.conv(f"{prefix}.mha.in_proj_weight", f"{prefix}.mha.in_proj_bias")
-        self.out_proj = pk.conv(f"{prefix}.mha.out_proj.weight", f"{prefix}.mha.out_proj.bias")
-        self.ff0 = pk.conv(f"{prefix}.ff.0.weight", f"{prefix}.ff.0.bias")
-        self.ff2 = pk.conv(f"{prefix}.ff.2.weight", f"{prefix}.ff.2.bias")
+        self.ln1 = (pk.vec(keys.ln1.weight), pk.vec(keys.ln1.bias))
+        self.ln2 = (pk.vec(keys.ln2.weight), pk.vec(keys.ln2.bias))
+        self.in_proj = pk.conv(*keys.in_proj)
+        self.out_proj = pk.conv(*keys.out_proj)
+        self.ff0 = pk.conv(*keys.ff0)
+        self.ff2 = pk.conv(*keys.ff2)
         # LayerNorm folded into the Linear layer behind it (tensor-core formats): ln1 -> in_proj, ln2 -> ff.0
         self.fold = pk.fmt != FMT_F32
         if self.fold:
-            self.in_proj_ln = pack_linear_ln(pk, f"{prefix}.mha.in_proj_weight", f"{prefix}.mha.in_proj_bias", f"{prefix}.ln1.weight",
-                                             f"{prefix}.ln1.bias")
-            self.ff0_ln = pack_linear_ln(pk, f"{prefix}.ff.0.weight", f"{prefix}.ff.0.bias", f"{prefix}.ln2.weight", f"{prefix}.ln2.bias")
+            self.in_proj_ln = pack_linear_ln(pk, *keys.in_proj, *keys.ln1)
+            self.ff0_ln = pack_linear_ln(pk, *keys.ff0, *keys.ln2)
 
 
 def attention_block(k: Kernels, aw: AttentionW, x: Act) -> Act:
@@ -521,6 +525,14 @@ class TimeProjector:
         self.b.append(b)
         self.set_of.append(torch.full((c,), set_idx, dtype=torch.int32, device=self.device))
 
+    def add_heads(self, heads: Sequence["TimeHead"], get: Callable[[str], torch.Tensor]) -> None:
+        """Add the layout's heads in column order; heads naming the same Fourier W share one set.  `get(key)`: a key's tensor."""
+        sets: Dict[str, int] = {}
+        for h in heads:
+            if h.fourier not in sets:
+                sets[h.fourier] = self.add_set(get(h.fourier))
+            self.add_head(h.name, sets[h.fourier], get(h.weight), get(h.bias))
+
     def finalize(self) -> None:
         self._packed = (torch.stack(self.sets).contiguous(), torch.cat(self.w).contiguous(),
                         torch.cat(self.b).contiguous(), torch.cat(self.set_of).contiguous())
@@ -549,39 +561,107 @@ class TimeProjector:
         return table[:, a:b]
 
 
+# -- checkpoint layout ----------------------------------------------------------------------------------------------------
+# The state-dict keys of the score-UNet (the reference's checkpoint format, mirrored by score_unet.py's module tree), as plain
+# records in forward order, under a key prefix: "" for a standalone module's own state dict.  Both engines read the network
+# through them, and keep their packed weights in records of the same types, under the same field names.
+Affine = namedtuple("Affine", "weight bias")                              # a convolution, Linear or normalisation layer
+BatchNormKeys = namedtuple("BatchNormKeys", "weight bias running_mean running_var")
+ConvBN = namedtuple("ConvBN", "conv bn")                                  # a convolution without bias + the BatchNorm2d behind it
+AttnKeys = namedtuple("AttnKeys", "ln1 in_proj out_proj ln2 ff0 ff2")     # ImageSelfAttention, in forward order
+# one SiLU -> Linear time projection: its TimeProjector head name, the key of its Fourier features' W, its Linear
+TimeHead = namedtuple("TimeHead", "name fourier weight bias")
+# a BasicBlock: ConvBN sites (down: the 1x1 downsample or None) and the stride of conv1 and the downsample
+EncBlock = namedtuple("EncBlock", "c1 c2 down stride")
+# stem: conv1.weight; attn: {stage: the AttnKeys behind it}; heads: enc0 (the stem) .. enc4 (stage 4), sharing one Fourier W
+EncoderLayout = namedtuple("EncoderLayout", "stem conv2 stages attn heads label_emb")
+# a DecoderBlock: conv_up is the resize convolution or the transposed convolution; n1 / n2: the GroupNorm's Affine, None for
+# InstanceNorm or nn.Identity; g1 / g2: the group counts (the channel count for InstanceNorm); head: its TimeHead
+DecBlock = namedtuple("DecBlock", "conv_up conv n1 n2 g1 g2 attn head")
+DecoderLayout = namedtuple("DecoderLayout", "blocks final_up final_conv")   # final_up: final_layer's up-path, as DecBlock.conv_up
+
+
+def _affine(p: str) -> Affine:
+    return Affine(f"{p}weight", f"{p}bias")
+
+
+def batchnorm_keys(p: str) -> BatchNormKeys:
+    return BatchNormKeys(f"{p}.weight", f"{p}.bias", f"{p}.running_mean", f"{p}.running_var")
+
+
+def attention_layout(p: str) -> AttnKeys:
+    return AttnKeys(_affine(f"{p}ln1."), Affine(f"{p}mha.in_proj_weight", f"{p}mha.in_proj_bias"), _affine(f"{p}mha.out_proj."),
+                    _affine(f"{p}ln2."), _affine(f"{p}ff.0."), _affine(f"{p}ff.2."))
+
+
+def encoder_layout(spec: "UNetSpec", p: str = "encoder.") -> EncoderLayout:
+    conv_bn = lambda conv, bn: ConvBN(f"{conv}weight", batchnorm_keys(bn))
+    stages, inplanes = [], FMAP_CHANNELS[0]
+    for li, nblk in enumerate(spec.block_layers, start=1):
+        planes, blocks = FMAP_CHANNELS[li], []
+        for b in range(nblk):
+            bp = f"{p}layer{li}.{b}."
+            stride = 2 if (b == 0 and li > 1) else 1
+            down = conv_bn(f"{bp}downsample.0.", f"{bp}downsample.1") if stride != 1 or inplanes != planes else None
+            blocks.append(EncBlock(conv_bn(f"{bp}conv1.", f"{bp}bn1"), conv_bn(f"{bp}conv2.", f"{bp}bn2"), down, stride))
+            inplanes = planes
+        stages.append(tuple(blocks))
+    heads = tuple(TimeHead(f"enc{i}", f"{p}sinusoidal_embedding.W", f"{p}time_projection_layers.{i}.1.weight",
+                           f"{p}time_projection_layers.{i}.1.bias") for i in range(len(FMAP_CHANNELS)))
+    return EncoderLayout(f"{p}conv1.weight", conv_bn(f"{p}conv2.", f"{p}bn1"), tuple(stages),
+                         {i: attention_layout(f"{p}attention_layers.{i}.") for i in (3, 4)}, heads,
+                         f"{p}label_emb.weight" if spec.has_labels else None)
+
+
+def _up_site(p: str, use_resize_conv: bool) -> Affine:
+    return _affine(f"{p}conv_up." if use_resize_conv else f"{p}transpose.")
+
+
+def decoder_block_layout(p: str, head: str, cin: int, cout: int, attn: bool, norm: str, gn_groups: int,
+                         use_resize_conv: bool) -> DecBlock:
+    group = norm == "group"
+    return DecBlock(_up_site(p, use_resize_conv), _affine(f"{p}conv."), _affine(f"{p}norm1.") if group else None,
+                    _affine(f"{p}norm2.") if group else None, max(1, min(gn_groups, cin)) if group else cin,
+                    max(1, min(gn_groups, cout)) if group else cout, attention_layout(f"{p}attention.") if attn else None,
+                    TimeHead(head, f"{p}sinusoidal_embedding.W", f"{p}time_projection_layer.1.weight", f"{p}time_projection_layer.1.bias"))
+
+
+def decoder_layout(spec: "UNetSpec", p: str = "decoder.") -> DecoderLayout:
+    """The final layer runs without a time input: its Fourier W and time projection are not part of the layout."""
+    blocks = tuple(decoder_block_layout(f"{p}residual_layers.{i}.", f"dec{i}", cin, cout, attn, spec.norm, spec.gn_groups,
+                                        spec.use_resize_conv) for i, (cin, cout, attn) in enumerate(spec.plan))
+    return DecoderLayout(blocks, _up_site(f"{p}final_layer.", spec.use_resize_conv), _affine(f"{p}final_layer.conv."))
+
+
+def stem_matrix(w1: torch.Tensor) -> torch.Tensor:              # conv1.weight [64][cin][8][8] -> the stem kernels' [cin][tap][co]
+    return w1.permute(1, 2, 3, 0).reshape(w1.shape[1], 64, 64).contiguous()
+
+
+def final_matrix(wf: torch.Tensor) -> torch.Tensor:             # final_layer.conv.weight [cout][cin][3][3] -> [cout][tap][cin]
+    return wf.permute(0, 2, 3, 1).reshape(wf.shape[0], 9, wf.shape[1]).contiguous()
+
+
 class EncoderEngine:
-    def __init__(self, sd, prefix: str, *, block_layers: Sequence[int], n_heads: int, te: int, has_labels: bool,
-                 fmt: int, device, tp: TimeProjector) -> None:
+    def __init__(self, sd, spec: "UNetSpec", lay: EncoderLayout, *, fmt: int, device, tp: TimeProjector) -> None:
         pk = _Packer(sd, fmt, device)
         self.k = Kernels(fmt, device)
-        self.fmt, self.device, self.prefix = fmt, device, prefix
-        p = prefix
-        w1 = pk.get(f"{p}conv1.weight")                                  # [64, cin, 8, 8]
+        self.fmt, self.device, self.tp = fmt, device, tp
+        w1 = pk.get(lay.stem)                                            # [64, cin, 8, 8]
         self.cin = w1.shape[1]
-        self.stem_w = w1.permute(1, 2, 3, 0).reshape(self.cin, 64, 64).contiguous()   # [cin][tap][co]
+        self.stem_w = stem_matrix(w1)
         if fmt != FMT_F32:
             # tensor-core stem: conv1 as a 1x1 convolution over the im2col tensor (K index = ci * 64 + r * 8 + s = OIHW order)
-            def km(wsub):
-                return pack_tc_matrix(wsub.reshape(64, -1).contiguous(), fmt)
+            km = lambda wsub: pack_tc_matrix(wsub.reshape(64, -1).contiguous(), fmt)
             self.stem_cw_all = ConvW(km(w1), None, self.cin * 64, 64, 1, 1)
             self.stem_cw_x = ConvW(km(w1[:, :1]), None, 64, 64, 1, 1)
-        self.conv2 = pk.conv(f"{p}conv2.weight", bn=f"{p}bn1")
-        self.layers = []
-        for li, nblk in enumerate(block_layers, start=1):
-            blocks = []
-            for b in range(nblk):
-                bp = f"{p}layer{li}.{b}"
-                stride = 2 if (b == 0 and li > 1) else 1
-                down = pk.conv(f"{bp}.downsample.0.weight", bn=f"{bp}.downsample.1") if f"{bp}.downsample.0.weight" in sd else None
-                blocks.append((pk.conv(f"{bp}.conv1.weight", bn=f"{bp}.bn1"), pk.conv(f"{bp}.conv2.weight", bn=f"{bp}.bn2"), down, stride))
-            self.layers.append(blocks)
-        self.attn = {i: AttentionW(pk, f"{p}attention_layers.{i}", n_heads) for i in (3, 4)}
-        set0 = tp.add_set(pk.get(f"{p}sinusoidal_embedding.W"))
-        for i in range(5):
-            tp.add_head(f"enc{i}", set0, pk.get(f"{p}time_projection_layers.{i}.1.weight"), pk.vec(f"{p}time_projection_layers.{i}.1.bias"))
-        if has_labels:
-            tp.label_emb = pk.get(f"{p}label_emb.weight").contiguous()
-        self.tp = tp
+        conv_bn = lambda s: pk.conv(s.conv, bn=s.bn)
+        self.conv2 = conv_bn(lay.conv2)
+        self.layers = [[s._replace(down=None if s.down is None else conv_bn(s.down), c1=conv_bn(s.c1), c2=conv_bn(s.c2))
+                        for s in stage] for stage in lay.stages]
+        self.attn = {i: AttentionW(pk, keys, spec.n_heads) for i, keys in lay.attn.items()}
+        tp.add_heads(lay.heads, pk.get)
+        if lay.label_emb is not None:
+            tp.label_emb = pk.get(lay.label_emb).contiguous()
 
     def alloc_partial(self, npl: int, h: int, w: int):
         """Buffer for `stem_partial`: fp32 NHWC tensor (fp32 mode) or an `Act` in the engine's format (tensor-core modes,
@@ -654,63 +734,44 @@ class EncoderEngine:
         return fmaps
 
 
+def pack_decoder_block(pk: _Packer, s: DecBlock, use_resize_conv: bool, n_heads: int) -> DecBlock:
+    norm = lambda a: (None, None) if a is None else (pk.vec(a.weight), pk.vec(a.bias))      # n1 / n2: (gamma, beta)
+    return s._replace(conv_up=pk.up(s.conv_up, use_resize_conv), conv=pk.conv(*s.conv), n1=norm(s.n1), n2=norm(s.n2),
+                      attn=None if s.attn is None else AttentionW(pk, s.attn, n_heads))
+
+
 class DecoderEngine:
-    def __init__(self, sd, prefix: str, *, plan: Sequence[Tuple[int, int, bool]], n_heads: int, norm: str,
-                 gn_groups: int, activation: str, use_resize_conv: bool, out_channels: int, fmt: int, device,
-                 tp: TimeProjector) -> None:
+    def __init__(self, sd, spec: "UNetSpec", lay: DecoderLayout, *, fmt: int, device, tp: TimeProjector) -> None:
         pk = _Packer(sd, fmt, device)
-        self.use_resize_conv = use_resize_conv
         self.k = Kernels(fmt, device)
-        self.fmt, self.device = fmt, device
-        self.act = ACTS[activation]
-        self.norm, self.gn_groups = norm, gn_groups
-        self.blocks = []
-        for i, (cin, cout, attn) in enumerate(plan):
-            bp = f"{prefix}residual_layers.{i}"
-            affine = norm == "group"
-            blk = dict(
-                conv_up=(pk.conv(f"{bp}.conv_up.weight", f"{bp}.conv_up.bias") if use_resize_conv else
-                         pk.conv_transpose(f"{bp}.transpose.weight", f"{bp}.transpose.bias")),
-                conv=pk.conv(f"{bp}.conv.weight", f"{bp}.conv.bias"),
-                n1=(pk.vec(f"{bp}.norm1.weight"), pk.vec(f"{bp}.norm1.bias")) if affine else (None, None),
-                n2=(pk.vec(f"{bp}.norm2.weight"), pk.vec(f"{bp}.norm2.bias")) if affine else (None, None),
-                g1=max(1, min(gn_groups, cin)) if affine else cin,
-                g2=max(1, min(gn_groups, cout)) if affine else cout,
-                attn=AttentionW(pk, f"{bp}.attention", n_heads) if attn else None,
-                name=f"dec{i}")
-            s = tp.add_set(pk.get(f"{bp}.sinusoidal_embedding.W"))
-            tp.add_head(f"dec{i}", s, pk.get(f"{bp}.time_projection_layer.1.weight"), pk.vec(f"{bp}.time_projection_layer.1.bias"))
-            self.blocks.append(blk)
-        fp = f"{prefix}final_layer"
-        self.final_up = (pk.conv(f"{fp}.conv_up.weight", f"{fp}.conv_up.bias") if use_resize_conv else
-                         pk.conv_transpose(f"{fp}.transpose.weight", f"{fp}.transpose.bias"))
-        wf = pk.get(f"{fp}.conv.weight")                                   # [cout, cin, 3, 3]
-        self.final_w = wf.permute(0, 2, 3, 1).reshape(wf.shape[0], 9, wf.shape[1]).contiguous()
-        self.final_b = pk.vec(f"{fp}.conv.bias")
-        self.out_channels = out_channels
-        self.tp = tp
+        self.fmt, self.device, self.tp = fmt, device, tp
+        self.use_resize_conv, self.out_channels, self.act = spec.use_resize_conv, spec.out_channels, ACTS[spec.activation]
+        self.blocks = [pack_decoder_block(pk, s, spec.use_resize_conv, spec.n_heads) for s in lay.blocks]
+        tp.add_heads([s.head for s in lay.blocks], pk.get)
+        self.final_up = pk.up(lay.final_up, spec.use_resize_conv)
+        self.final_w = final_matrix(pk.get(lay.final_conv.weight))
+        self.final_b = pk.vec(lay.final_conv.bias)
 
     def forward(self, fmaps: List[Act], tproj: torch.Tensor, inv_std: InvStd, dst: Optional[torch.Tensor] = None) -> torch.Tensor:
         k, tp = self.k, self.tp
         rev = list(reversed(fmaps))
         out = rev[0]
         for i, blk in enumerate(self.blocks):
-            if self.use_resize_conv and k.up_fused_ok(out, blk["conv_up"]):
-                a, st1 = k.conv_up_fused(out, blk["conv_up"], gn_stats=True)       # the bilinear upsample inside the operand stage
+            if self.use_resize_conv and k.up_fused_ok(out, blk.conv_up):
+                a, st1 = k.conv_up_fused(out, blk.conv_up, gn_stats=True)       # the bilinear upsample inside the operand stage
             elif self.use_resize_conv:
                 up = k.upsample2x(out)
-                a, st1 = k.conv(up, blk["conv_up"], pad=1, gn_stats=True)
+                a, st1 = k.conv(up, blk.conv_up, pad=1, gn_stats=True)
             else:
-                a, st1 = k.conv_transpose2x(out, blk["conv_up"]), None
-            a = k.groupnorm(a, *blk["n1"], groups=blk["g1"], stats=st1)
-            b, st2 = k.conv(a, blk["conv"], pad=1, gn_stats=True)
+                a, st1 = k.conv_transpose2x(out, blk.conv_up), None
+            a = k.groupnorm(a, *blk.n1, groups=blk.g1, stats=st1)
+            b, st2 = k.conv(a, blk.conv, pad=1, gn_stats=True)
             skip = rev[i + 1]
             if (skip.n, skip.h, skip.w, skip.c) != (b.n, b.h, b.w, b.c):
                 raise AssertionError(f"prev_fmap shape {(skip.n, skip.c, skip.h, skip.w)} must match output shape {(b.n, b.c, b.h, b.w)}")
-            out = k.groupnorm(b, *blk["n2"], groups=blk["g2"], act=self.act, skip=skip, tproj=tp.cols(tproj, blk["name"]),
-                              stats=st2)
-            if blk["attn"] is not None:
-                out = attention_block(k, blk["attn"], out)
+            out = k.groupnorm(b, *blk.n2, groups=blk.g2, act=self.act, skip=skip, tproj=tp.cols(tproj, blk.head.name), stats=st2)
+            if blk.attn is not None:
+                out = attention_block(k, blk.attn, out)
         # the final layer: conv_up's output `a` for the final convolution, or the final 64 -> 1 convolution's per-tap partial
         # products `pr` out of conv_up's epilogue (its 64-channel output never reaches HBM; tc_common.cuh: projection epilogue)
         a = pr = None
@@ -751,7 +812,6 @@ def concat_planes(x_batch: int, lsm, topo, cond, device) -> Optional[torch.Tenso
 @dataclass
 class UNetSpec:
     """Architecture knobs recovered from the module tree (they mirror the reference constructors)."""
-    cin_total: int
     time_embedding: int = 256
     block_layers: Tuple[int, ...] = (2, 2, 2, 2)
     n_heads: int = 4
@@ -784,12 +844,8 @@ class UNetEngine:
         self.fmt = PRECISIONS[precision]
         with torch.cuda.device(device), torch.no_grad():
             self.tp = TimeProjector(device, spec.time_embedding)
-            self.enc = EncoderEngine(sd, "encoder.", block_layers=spec.block_layers, n_heads=spec.n_heads,
-                                     te=spec.time_embedding, has_labels=spec.has_labels, fmt=self.fmt, device=device, tp=self.tp)
-            self.dec = DecoderEngine(sd, "decoder.", plan=spec.plan, n_heads=spec.n_heads, norm=spec.norm,
-                                     gn_groups=spec.gn_groups, activation=spec.activation,
-                                     use_resize_conv=spec.use_resize_conv, out_channels=spec.out_channels, fmt=self.fmt,
-                                     device=device, tp=self.tp)
+            self.enc = EncoderEngine(sd, spec, encoder_layout(spec), fmt=self.fmt, device=device, tp=self.tp)
+            self.dec = DecoderEngine(sd, spec, decoder_layout(spec), fmt=self.fmt, device=device, tp=self.tp)
             self.tp.finalize()
 
     def check_input(self, x: torch.Tensor) -> None:

@@ -26,7 +26,6 @@ from ._lib import call
 logger = logging.getLogger(__name__)
 
 DEFAULT_PRECISION = os.environ.get("SBGM_B200_PRECISION", "bf16x3")
-_FMAPS = (64, 64, 128, 256, 512)
 
 
 def _default_device(device=None) -> torch.device:
@@ -109,8 +108,8 @@ class ImageSelfAttention(nn.Module):
 
         def build(dev):
             fmt = _eng.PRECISIONS[self.precision]
-            sd = {f"a.{k}": v for k, v in self.state_dict().items()}
-            return _eng.Kernels(fmt, dev), _eng.AttentionW(_eng._Packer(sd, fmt, dev), "a", self.n_heads), fmt
+            return _eng.Kernels(fmt, dev), _eng.AttentionW(_eng._Packer(self.state_dict(), fmt, dev), _eng.attention_layout(""),
+                                                           self.n_heads), fmt
 
         with torch.no_grad(), torch.cuda.device(self.ln1.weight.device):
             k, aw, fmt = self._cache.get(self, self.precision, build)
@@ -167,8 +166,8 @@ class Encoder(nn.Module):
                 inplanes = planes
             setattr(self, f"layer{li}", nn.Sequential(*blocks))
         self.sinusoidal_embedding = SinusoidalEmbedding(time_embedding)
-        self.time_projection_layers = self.make_time_projections(_FMAPS)
-        self.attention_layers = self.make_attention_layers(_FMAPS)
+        self.time_projection_layers = self.make_time_projections(_eng.FMAP_CHANNELS)
+        self.attention_layers = self.make_attention_layers(_eng.FMAP_CHANNELS)
         self.conv2 = nn.Conv2d(64, 64, kernel_size=(8, 8), stride=(2, 2), padding=(3, 3), bias=False)
         if num_classes is not None:
             self.label_emb = nn.Embedding(num_classes + 1, time_embedding)
@@ -185,13 +184,15 @@ class Encoder(nn.Module):
         return nn.ModuleList([ImageSelfAttention(ch, self.n_heads) if i >= len(chans) - 2 else nn.Identity()
                               for i, ch in enumerate(chans)])
 
+    def _spec(self) -> _eng.UNetSpec:                       # the encoder's fields (the decoder's keep their defaults, unread)
+        return _eng.UNetSpec(time_embedding=self.time_embedding, block_layers=tuple(self.block_layers), n_heads=self.n_heads,
+                             has_labels=self.num_classes is not None)
+
     def _engine(self):
         def build(dev):
-            fmt = _eng.PRECISIONS[self.precision]
             tp = _eng.TimeProjector(dev, self.time_embedding)
-            sd = {f"encoder.{k}": v for k, v in self.state_dict().items()}
-            enc = _eng.EncoderEngine(sd, "encoder.", block_layers=self.block_layers, n_heads=self.n_heads,
-                                     te=self.time_embedding, has_labels=self.num_classes is not None, fmt=fmt,
+            spec = self._spec()
+            enc = _eng.EncoderEngine(self.state_dict(), spec, _eng.encoder_layout(spec, ""), fmt=_eng.PRECISIONS[self.precision],
                                      device=dev, tp=tp)
             tp.finalize()
             return enc
@@ -208,11 +209,8 @@ class Encoder(nn.Module):
             # feature maps; gradients flow through ScoreNet.forward / loss_fn, which own the backward tape.
             from .train_engine import TrainEngine
             with torch.no_grad(), torch.cuda.device(dev):
-                tensors = {f"encoder.{k}": v for k, v in list(self.named_parameters()) + list(self.named_buffers())}
-                spec = _eng.UNetSpec(cin_total=self.input_channels, time_embedding=self.time_embedding,
-                                     block_layers=tuple(self.block_layers), n_heads=self.n_heads,
-                                     has_labels=self.num_classes is not None)
-                eng = TrainEngine(tensors, spec, self.precision, dev, bn_train=True, encoder_only=True)
+                tensors = dict(list(self.named_parameters()) + list(self.named_buffers()))
+                eng = TrainEngine(tensors, self._spec(), self.precision, dev, bn_train=True, encoder_only=True)
                 planes = _eng.concat_planes(x.shape[0], lsm_cond, topo_cond, cond_img, dev)
                 if planes is not None and planes.shape[0] != x.shape[0]:
                     planes = planes.expand(x.shape[0], -1, -1, -1).contiguous()
@@ -276,67 +274,52 @@ class DecoderBlock(nn.Module):
 
         def build(d):
             fmt = _eng.PRECISIONS[self.precision]
+            pk = _eng._Packer(self.state_dict(), fmt, d)
+            s = _eng.decoder_block_layout("", "dec0", self.input_channels, self.output_channels, self.compute_attn, self.norm_kind,
+                                          self.gn_groups, self.use_resize_conv)
+            s = s._replace(n1=None if id1 else s.n1, n2=None if id2 else s.n2)      # an Identity norm (Decoder.final_layer) has no keys
             tp = _eng.TimeProjector(d, self.time_embedding)
-            own = dict(self.state_dict())
-            for nm, c, ident in (("norm1", self.input_channels, id1), ("norm2", self.output_channels, id2)):
-                if ident and self.norm_kind == "group":      # an Identity norm (Decoder.final_layer): placeholders, never applied
-                    own[f"{nm}.weight"] = torch.ones(c, device=d)
-                    own[f"{nm}.bias"] = torch.zeros(c, device=d)
-            sd = {f"d.residual_layers.0.{k}": v for k, v in own.items()}
-            # a one-block decoder without final layer: reuse DecoderEngine's block packing
-            sd.update({f"d.final_layer.{k}": v for k, v in own.items() if k.startswith(("conv_up", "transpose", "conv."))})
-            sd["d.final_layer.conv.weight"] = self.conv.weight[:1]
-            sd["d.final_layer.conv.bias"] = self.conv.bias[:1]
-            de = _eng.DecoderEngine(sd, "d.", plan=[(self.input_channels, self.output_channels, self.compute_attn)],
-                                    n_heads=self.n_heads, norm=self.norm_kind, gn_groups=self.gn_groups,
-                                    activation=_act_name(self.activation), use_resize_conv=self.use_resize_conv,
-                                    out_channels=1, fmt=fmt, device=d, tp=tp)
+            tp.add_heads([s.head], pk.get)
             tp.finalize()
-            return de, fmt
+            blk = _eng.pack_decoder_block(pk, s, self.use_resize_conv, self.n_heads)
+            return _eng.Kernels(fmt, d), blk, tp, pk.conv(s.head.weight, s.head.bias), fmt
 
         with torch.no_grad(), torch.cuda.device(dev):
-            de, fmt = self._cache.get(self, (self.precision, id1, id2), build)
+            k, blk, tp, tlin, fmt = self._cache.get(self, (self.precision, id1, id2), build)
+            act = _eng.ACTS[_act_name(self.activation)]
             out_shape = (fmap.shape[0], self.output_channels, 2 * fmap.shape[2], 2 * fmap.shape[3])
             skip = None
             if prev_fmap is not None and torch.is_tensor(prev_fmap):
                 if tuple(prev_fmap.shape) != out_shape:
                     raise AssertionError(f"prev_fmap shape {tuple(prev_fmap.shape)} must match output shape {out_shape}")
                 skip = _eng.Act.from_nchw(prev_fmap.to(dev), fmt)
-            k, blk = de.k, de.blocks[0]
             tcols = None
             if t is not None:
                 t = t.to(dev)
                 if t.dim() == 1 or (t.dim() == 2 and t.shape[-1] != self.time_embedding):      # raw timesteps [B]
-                    tcols = de.tp.cols(de.tp(t.reshape(-1).float(), None), "dec0")
+                    tcols = tp.cols(tp(t.reshape(-1).float(), None), blk.head.name)
                 else:                                   # a precomputed embedding [B, time_dim]: SiLU -> Linear on the kernels
-                    tcols = self._project_embedding(k, t.float(), fmt)
+                    tcols = self._project_embedding(k, tlin, t.float(), fmt)
             x = _eng.Act.from_nchw(fmap.to(dev), fmt)
-            a = k.conv(k.upsample2x(x), blk["conv_up"], pad=1) if self.use_resize_conv else k.conv_transpose2x(x, blk["conv_up"])
+            a = k.conv(k.upsample2x(x), blk.conv_up, pad=1) if self.use_resize_conv else k.conv_transpose2x(x, blk.conv_up)
             if not id1:
-                a = k.groupnorm(a, *blk["n1"], groups=blk["g1"])
-            b = k.conv(a, blk["conv"], pad=1)
+                a = k.groupnorm(a, *blk.n1, groups=blk.g1)
+            b = k.conv(a, blk.conv, pad=1)
             if id2:
-                out = k.affine(b, skip=skip, tproj=tcols, act=de.act)            # x + prev_fmap + t_proj, then the activation
+                out = k.affine(b, skip=skip, tproj=tcols, act=act)            # x + prev_fmap + t_proj, then the activation
             else:
-                out = k.groupnorm(b, *blk["n2"], groups=blk["g2"], act=de.act, skip=skip, tproj=tcols)
-            if blk["attn"] is not None:
-                out = _eng.attention_block(k, blk["attn"], out)
+                out = k.groupnorm(b, *blk.n2, groups=blk.g2, act=act, skip=skip, tproj=tcols)
+            if blk.attn is not None:
+                out = _eng.attention_block(k, blk.attn, out)
             return out.to_nchw()
 
-    def _project_embedding(self, k, t_emb: torch.Tensor, fmt: int) -> torch.Tensor:
-        """time_projection_layer (SiLU -> Linear) of a precomputed embedding [B, time_dim] -> fp32 [B, C_out]."""
-        cache = self.__dict__.setdefault("_tproj_cw", {})
-        lin = self.time_projection_layer[1]
-        key = (fmt, lin.weight._version, lin.bias._version, lin.weight.data_ptr())
-        if key not in cache:
-            cache.clear()
-            pk = _eng._Packer({"w": lin.weight.detach(), "b": lin.bias.detach()}, fmt, lin.weight.device)
-            cache[key] = pk.conv("w", "b")
+    def _project_embedding(self, k, lin: _eng.ConvW, t_emb: torch.Tensor, fmt: int) -> torch.Tensor:
+        """time_projection_layer (SiLU -> `lin`, its packed Linear) of a precomputed embedding [B, time_dim] -> fp32 [B, C_out]."""
         rows = t_emb.shape[0]
         tok = _eng.Act.from_nchw(t_emb.t().reshape(1, self.time_embedding, 1, rows).contiguous(), fmt)
         h = tok.like()
         _eng.call("sbgm_act_forward", tok.ptr, tok.plane, h.ptr, h.plane, fmt, tok.plane, _eng.ACTS["silu"], _eng._stream())
-        out = k.linear(h, cache[key])
+        out = k.linear(h, lin)
         return out.to_nchw().reshape(self.output_channels, rows).t().contiguous()
 
 
@@ -379,11 +362,10 @@ class Decoder(nn.Module):
         def build(dev):
             fmt = _eng.PRECISIONS[self.precision]
             tp = _eng.TimeProjector(dev, self.time_embedding)
-            sd = {f"decoder.{k}": v for k, v in self.state_dict().items()}
-            dec = _eng.DecoderEngine(sd, "decoder.", plan=self.plan(), n_heads=self.n_heads, norm=self.norm,
-                                     gn_groups=self.gn_groups, activation=_act_name(self.activation),
-                                     use_resize_conv=self.use_resize_conv, out_channels=self.output_channels, fmt=fmt,
-                                     device=dev, tp=tp)
+            spec = _eng.UNetSpec(time_embedding=self.time_embedding, n_heads=self.n_heads, plan=self.plan(),
+                                 out_channels=self.output_channels, use_resize_conv=self.use_resize_conv, norm=self.norm,
+                                 gn_groups=self.gn_groups, activation=_act_name(self.activation))
+            dec = _eng.DecoderEngine(self.state_dict(), spec, _eng.decoder_layout(spec, ""), fmt=fmt, device=dev, tp=tp)
             tp.finalize()
             return dec, fmt
         return self._cache.get(self, self.precision, build)
@@ -420,10 +402,9 @@ class ScoreNet(nn.Module):
 
     def spec(self) -> _eng.UNetSpec:
         e, d = self.encoder, self.decoder
-        return _eng.UNetSpec(cin_total=e.input_channels, time_embedding=e.time_embedding, block_layers=tuple(e.block_layers),
-                             n_heads=e.n_heads, has_labels=e.num_classes is not None, plan=d.plan(),
-                             out_channels=d.output_channels, use_resize_conv=d.use_resize_conv, norm=d.norm,
-                             gn_groups=d.gn_groups, activation=_act_name(d.activation))
+        return _eng.UNetSpec(time_embedding=e.time_embedding, block_layers=tuple(e.block_layers), n_heads=e.n_heads,
+                             has_labels=e.num_classes is not None, plan=d.plan(), out_channels=d.output_channels,
+                             use_resize_conv=d.use_resize_conv, norm=d.norm, gn_groups=d.gn_groups, activation=_act_name(d.activation))
 
     def engine(self) -> _eng.UNetEngine:
         """Packed-weight engine for the current parameters (cached; rebuilt after parameter updates)."""

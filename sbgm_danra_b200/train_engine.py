@@ -21,8 +21,9 @@ import torch
 from . import _lib
 from ._capture import graph_capture
 from ._lib import ACT_GELU, ACT_NONE, ACT_RELU, FMT_BF16X2, FMT_F32, call
-from .engine import (ACTS, BN_EPS, GN_EPS, LN_EPS, PRECISIONS, Act, ConvW, InvStd, Kernels, UNetSpec, _ptr, _stream, engine_device,
-                     pack_transpose)
+from .engine import (ACTS, BN_EPS, GN_EPS, LN_EPS, PRECISIONS, Act, Affine, AttnKeys, ConvBN, ConvW, DecBlock, InvStd, Kernels,
+                     TimeProjector, UNetSpec, _ptr, _stream, decoder_layout, encoder_layout, engine_device, final_matrix,
+                     pack_transpose, stem_matrix)
 
 BN_MOMENTUM = 0.1
 # "fp16x2" is an inference storage format (engine.py); a model set to it trains on the bf16x3 kernels
@@ -498,29 +499,22 @@ class TrainKernels:
         return y
 
 
-class _AttnLayers:
-    def __init__(self, sd, prefix: str, heads: int, fmt: int, plan: Optional[PackPlan] = None) -> None:
-        g = lambda k: sd[f"{prefix}.{k}"]
-        lin = lambda w, b_: ConvLayer(f"{prefix}.{w}", g(w), g(b_), fmt, f"{prefix}.{b_}", plan=plan)
-        self.heads, self.prefix = heads, prefix
-        self.ln1 = (g("ln1.weight"), g("ln1.bias"))
-        self.ln2 = (g("ln2.weight"), g("ln2.bias"))
-        self.in_proj = lin("mha.in_proj_weight", "mha.in_proj_bias")
-        self.out_proj = lin("mha.out_proj.weight", "mha.out_proj.bias")
-        self.ff0 = lin("ff.0.weight", "ff.0.bias")
-        self.ff2 = lin("ff.2.weight", "ff.2.bias")
+def _attn_layers(sd, keys: AttnKeys, fmt: int, plan: PackPlan) -> AttnKeys:
+    """An attention block under its layout's field names: ConvLayers, and (gamma, beta, gamma name, beta name) per LayerNorm."""
+    lin = lambda a: ConvLayer(a.weight, sd[a.weight], sd[a.bias], fmt, a.bias, plan=plan)
+    ln = lambda a: (sd[a.weight], sd[a.bias], *a)
+    return AttnKeys(ln(keys.ln1), lin(keys.in_proj), lin(keys.out_proj), ln(keys.ln2), lin(keys.ff0), lin(keys.ff2))
 
 
-def _attention_block(tk: TrainKernels, aw: _AttnLayers, x: Act) -> Act:
+def _attention_block(tk: TrainKernels, aw: AttnKeys, heads: int, x: Act) -> Act:
     """ImageSelfAttention.forward (score_unet.py:136-148) with its backward recorded."""
     tok = x.tokens()
     b, s, c = x.n, x.h * x.w, x.c
-    p = aw.prefix
-    h1 = tk.layernorm(tok, *aw.ln1, f"{p}.ln1.weight", f"{p}.ln1.bias")
+    h1 = tk.layernorm(tok, *aw.ln1)
     qkv = tk.conv(h1, aw.in_proj)
-    att = tk.attention_core(qkv, b, s, c, aw.heads)
+    att = tk.attention_core(qkv, b, s, c, heads)
     h = tk.conv(att, aw.out_proj, residual=tok)
-    g = tk.layernorm(h, *aw.ln2, f"{p}.ln2.weight", f"{p}.ln2.bias")
+    g = tk.layernorm(h, *aw.ln2)
     g1 = tk.conv(g, aw.ff0)
     g2 = tk.activation(g1, ACT_GELU)
     return tk.conv(g2, aw.ff2, residual=h).view(x.n, x.h, x.w, x.c)
@@ -534,11 +528,13 @@ class TrainEngine:
 
     def __init__(self, params: Dict[str, torch.Tensor], spec: UNetSpec, precision: str, device, bn_train: bool,
                  encoder_only: bool = False) -> None:
-        """`encoder_only`: `params` holds the encoder alone and `forward` returns its five feature maps (the standalone
-        `Encoder.forward` in .train(): batch statistics, running statistics updated; nothing is differentiated)."""
+        """`encoder_only`: `params` is the standalone Encoder's own state dict and `forward` returns its five feature maps
+        (`Encoder.forward` in .train(): batch statistics, running statistics updated; nothing is differentiated)."""
         device = engine_device(precision, device)
         self.spec, self.device, self.fmt, self.bn_train = spec, device, TRAIN_PRECISIONS[precision], bn_train
         self.encoder_only = encoder_only
+        self.enc_layout = encoder_layout(spec, "") if encoder_only else encoder_layout(spec)
+        self.dec_layout = None if encoder_only else decoder_layout(spec)
         self.sd = {k: v.detach() for k, v in params.items()}
         for k, v in self.sd.items():
             if v.is_floating_point() and (v.dtype != torch.float32 or not v.is_cuda):
@@ -566,84 +562,52 @@ class TrainEngine:
         self.touched[name] = g
         return g
 
-    def _bn(self, prefix: str) -> dict:
-        return dict(weight=self.sd[f"{prefix}.weight"], bias=self.sd[f"{prefix}.bias"], running_mean=self.sd[f"{prefix}.running_mean"],
-                    running_var=self.sd[f"{prefix}.running_var"], weight_name=f"{prefix}.weight", bias_name=f"{prefix}.bias")
-
     def _conv(self, wname: str, bname: Optional[str] = None, stride: int = 1, pad: int = 0) -> ConvLayer:
         return ConvLayer(wname, self.sd[wname], None if bname is None else self.sd[bname], self.fmt, bname, plan=self.plan,
                          stride=stride, pad=pad)
 
+    def _conv_bn(self, s: ConvBN, stride: int, pad: int) -> ConvBN:
+        bn = {field: self.sd[key] for field, key in s.bn._asdict().items()}          # weight, bias, running_mean, running_var
+        return ConvBN(self._conv(s.conv, stride=stride, pad=pad), dict(bn, weight_name=s.bn.weight, bias_name=s.bn.bias))
+
+    def _up(self, s: Affine):
+        return (self._conv(*s, 1, 1) if self.spec.use_resize_conv else
+                ConvTLayer(s.weight, self.sd[s.weight], self.sd[s.bias], self.fmt, s.bias))
+
+    def _dec_block(self, s: DecBlock) -> DecBlock:
+        norm = lambda a: (None,) * 4 if a is None else (self.sd[a.weight], self.sd[a.bias], *a)      # gamma, beta and their names
+        return s._replace(conv_up=self._up(s.conv_up), conv=self._conv(*s.conv, 1, 1), n1=norm(s.n1), n2=norm(s.n2),
+                          attn=None if s.attn is None else _attn_layers(self.sd, s.attn, self.fmt, self.plan))
+
     def _pack(self) -> None:
-        sd, spec, fmt = self.sd, self.spec, self.fmt
+        sd, spec, fmt, enc = self.sd, self.spec, self.fmt, self.enc_layout
         self.plan = PackPlan(fmt)
-        p = "encoder."
-        w1 = sd[f"{p}conv1.weight"]
+        w1 = sd[enc.stem]
         self.cin = w1.shape[1]
-        self.stem_w = w1.permute(1, 2, 3, 0).reshape(self.cin, 64, 64).contiguous()
+        self.stem_w = stem_matrix(w1)
         if fmt != FMT_F32:   # tensor-core stem: 1x1 convolution over the im2col tensor; [co][ci*64 + tap] IS conv1.weight's OIHW order
-            self.stem_layer = ConvLayer(f"{p}conv1.weight", w1.reshape(64, self.cin * 64, 1, 1), None, fmt, plan=self.plan, need_dx=False)
+            self.stem_layer = ConvLayer(enc.stem, w1.reshape(64, self.cin * 64, 1, 1), None, fmt, plan=self.plan, need_dx=False)
             self.stem_layer.shape = tuple(w1.shape)
-        self.conv2 = self._conv(f"{p}conv2.weight", stride=2, pad=3)
-        self.bn1 = self._bn(f"{p}bn1")
-        self.layers = []
-        for li, nblk in enumerate(spec.block_layers, start=1):
-            blocks = []
-            for b in range(nblk):
-                bp = f"{p}layer{li}.{b}"
-                stride = 2 if (b == 0 and li > 1) else 1
-                down = None
-                if f"{bp}.downsample.0.weight" in sd:
-                    down = (self._conv(f"{bp}.downsample.0.weight", stride=stride, pad=0), self._bn(f"{bp}.downsample.1"))
-                blocks.append(dict(c1=self._conv(f"{bp}.conv1.weight", stride=stride, pad=1), b1=self._bn(f"{bp}.bn1"),
-                                   c2=self._conv(f"{bp}.conv2.weight", stride=1, pad=1),
-                                   b2=self._bn(f"{bp}.bn2"), down=down, stride=stride))
-            self.layers.append(blocks)
-        self.enc_attn = {i: _AttnLayers(sd, f"{p}attention_layers.{i}", spec.n_heads, fmt, self.plan) for i in (3, 4)}
+        self.conv2, self.bn1 = self._conv_bn(enc.conv2, 2, 3)
+        self.layers = [[s._replace(down=None if s.down is None else self._conv_bn(s.down, s.stride, 0), c1=self._conv_bn(s.c1, s.stride, 1),
+                                   c2=self._conv_bn(s.c2, 1, 1)) for s in stage] for stage in enc.stages]
+        self.enc_attn = {i: _attn_layers(sd, keys, fmt, self.plan) for i, keys in enc.attn.items()}
         # time projector: same packing as inference (engine.TimeProjector) plus the names for the gradients
-        from .engine import TimeProjector
+        self.tp_heads = enc.heads + (() if self.encoder_only else tuple(s.head for s in self.dec_layout.blocks))
         self.tp = TimeProjector(self.device, spec.time_embedding)
-        self.tp_names: List[Tuple[str, str, int]] = []      # (weight name, bias name, channels) in head order
-        set0 = self.tp.add_set(sd[f"{p}sinusoidal_embedding.W"])
-        for i in range(5):
-            wn, bn = f"{p}time_projection_layers.{i}.1.weight", f"{p}time_projection_layers.{i}.1.bias"
-            self.tp.add_head(f"enc{i}", set0, sd[wn], sd[bn])
-            self.tp_names.append((wn, bn, sd[wn].shape[0]))
-        self.label_name = f"{p}label_emb.weight" if spec.has_labels else None
-        if spec.has_labels:
-            self.tp.label_emb = sd[self.label_name].contiguous()
-        self.act = ACTS[spec.activation]
-        if self.encoder_only:
-            self.tp.finalize()
-            self.plan.run()
-            return
-        d = "decoder."
-        affine = spec.norm == "group"
-        self.dec_blocks = []
-        for i, (cin, cout, attn) in enumerate(spec.plan):
-            bp = f"{d}residual_layers.{i}"
-            up_layer = (self._conv(f"{bp}.conv_up.weight", f"{bp}.conv_up.bias", 1, 1) if spec.use_resize_conv else
-                        ConvTLayer(f"{bp}.transpose.weight", sd[f"{bp}.transpose.weight"], sd[f"{bp}.transpose.bias"], fmt, f"{bp}.transpose.bias"))
-            blk = dict(conv_up=up_layer, conv=self._conv(f"{bp}.conv.weight", f"{bp}.conv.bias", 1, 1),
-                       n1=(sd[f"{bp}.norm1.weight"], sd[f"{bp}.norm1.bias"], f"{bp}.norm1.weight", f"{bp}.norm1.bias") if affine else (None, None, None, None),
-                       n2=(sd[f"{bp}.norm2.weight"], sd[f"{bp}.norm2.bias"], f"{bp}.norm2.weight", f"{bp}.norm2.bias") if affine else (None, None, None, None),
-                       g1=max(1, min(spec.gn_groups, cin)) if affine else cin, g2=max(1, min(spec.gn_groups, cout)) if affine else cout,
-                       attn=_AttnLayers(sd, f"{bp}.attention", spec.n_heads, fmt, self.plan) if attn else None, name=f"dec{i}")
-            s = self.tp.add_set(sd[f"{bp}.sinusoidal_embedding.W"])
-            wn, bn = f"{bp}.time_projection_layer.1.weight", f"{bp}.time_projection_layer.1.bias"
-            self.tp.add_head(f"dec{i}", s, sd[wn], sd[bn])
-            self.tp_names.append((wn, bn, sd[wn].shape[0]))
-            self.dec_blocks.append(blk)
+        self.tp.add_heads(self.tp_heads, sd.__getitem__)
+        if enc.label_emb is not None:
+            self.tp.label_emb = sd[enc.label_emb].contiguous()
         self.tp.finalize()
-        fp = f"{d}final_layer"
-        self.final_up = (self._conv(f"{fp}.conv_up.weight", f"{fp}.conv_up.bias", 1, 1) if spec.use_resize_conv else
-                         ConvTLayer(f"{fp}.transpose.weight", sd[f"{fp}.transpose.weight"], sd[f"{fp}.transpose.bias"], fmt, f"{fp}.transpose.bias"))
-        wf = sd[f"{fp}.conv.weight"]
-        if wf.shape[0] != 1:
-            raise NotImplementedError("the training path supports output_channels == 1 (the reference's only configuration)")
-        self.final_w = wf.permute(0, 2, 3, 1).reshape(wf.shape[0], 9, wf.shape[1]).contiguous()
-        self.final_b = sd[f"{fp}.conv.bias"].contiguous()
-        self.final_names = (f"{fp}.conv.weight", f"{fp}.conv.bias")
+        self.act = ACTS[spec.activation]
+        if (dec := self.dec_layout) is not None:
+            self.dec_blocks = [self._dec_block(s) for s in dec.blocks]
+            self.final_up = self._up(dec.final_up)
+            wf = sd[dec.final_conv.weight]
+            if wf.shape[0] != 1:
+                raise NotImplementedError("the training path supports output_channels == 1 (the reference's only configuration)")
+            self.final_w = final_matrix(wf)
+            self.final_b = sd[dec.final_conv.bias].contiguous()
         self.plan.run()            # every forward / data-gradient pack of the step: one batched launch
 
     # -- forward ----------------------------------------------------------------------------------------
@@ -691,7 +655,7 @@ class TrainEngine:
             if df is None:
                 return
             tk.channel_sums(df, dtproj=col(dtproj, "enc0"))
-            dw = self._param_grad("encoder.conv1.weight", (64, self.cin, 8, 8))
+            dw = self._param_grad(self.enc_layout.stem, (64, self.cin, 8, 8))
             ws2 = tk.scratch("stem", _lib.query("sbgm_stem_wgrad_workspace_floats", self.cin))
             call("sbgm_stem_wgrad", x.data_ptr(), _ptr(planes), 1 if planes is None else planes.shape[0], cc, df.ptr, df.plane, fmt,
                  dw.data_ptr(), n, h, w, ws2.data_ptr(), _stream())
@@ -707,15 +671,15 @@ class TrainEngine:
         for li, blocks in enumerate(self.layers, start=1):
             for bi, blk in enumerate(blocks):
                 last = bi == len(blocks) - 1
-                if blk["down"] is not None:
-                    idn = tk.batchnorm(tk.conv(hcur, blk["down"][0], stride=blk["stride"], pad=0), blk["down"][1], self.bn_train)
+                if blk.down is not None:
+                    idn = tk.batchnorm(tk.conv(hcur, blk.down.conv, stride=blk.stride, pad=0), blk.down.bn, self.bn_train)
                 else:
                     idn = hcur
-                mid = tk.batchnorm(tk.conv(hcur, blk["c1"], stride=blk["stride"], pad=1), blk["b1"], self.bn_train, act=ACT_RELU)
-                hcur = tk.batchnorm(tk.conv(mid, blk["c2"], stride=1, pad=1), blk["b2"], self.bn_train, act=ACT_RELU, residual=idn,
+                mid = tk.batchnorm(tk.conv(hcur, blk.c1.conv, stride=blk.stride, pad=1), blk.c1.bn, self.bn_train, act=ACT_RELU)
+                hcur = tk.batchnorm(tk.conv(mid, blk.c2.conv, stride=1, pad=1), blk.c2.bn, self.bn_train, act=ACT_RELU, residual=idn,
                                     tproj=col(tproj, f"enc{li}") if last else None, dtproj=col(dtproj, f"enc{li}") if last else None)
             if li in self.enc_attn:
-                hcur = _attention_block(tk, self.enc_attn[li], hcur)
+                hcur = _attention_block(tk, self.enc_attn[li], self.spec.n_heads, hcur)
             fmaps.append(hcur)
         if self.encoder_only:                  # standalone Encoder.forward: the feature maps are the result, no backward follows
             self.tape = tk.tape = None
@@ -728,18 +692,18 @@ class TrainEngine:
         for i, blk in enumerate(self.dec_blocks):
             # the two convolutions' bias gradients come out of the normalisation backward behind them (closed form)
             if self.spec.use_resize_conv:
-                a, st1 = tk.conv(tk.upsample2x(out), blk["conv_up"], pad=1, gn_stats=True, bias_grad=False)
-                a = tk.groupnorm(a, *blk["n1"], groups=blk["g1"], fused=st1, prev_bias=blk["conv_up"].bias_name)
+                a, st1 = tk.conv(tk.upsample2x(out), blk.conv_up, pad=1, gn_stats=True, bias_grad=False)
+                a = tk.groupnorm(a, *blk.n1, groups=blk.g1, fused=st1, prev_bias=blk.conv_up.bias_name)
             else:
-                a = tk.groupnorm(tk.conv_transpose2x(out, blk["conv_up"]), *blk["n1"], groups=blk["g1"])
-            b, st2 = tk.conv(a, blk["conv"], pad=1, gn_stats=True, bias_grad=False)
+                a = tk.groupnorm(tk.conv_transpose2x(out, blk.conv_up), *blk.n1, groups=blk.g1)
+            b, st2 = tk.conv(a, blk.conv, pad=1, gn_stats=True, bias_grad=False)
             skip = rev[i + 1]
             if (skip.n, skip.h, skip.w, skip.c) != (b.n, b.h, b.w, b.c):
                 raise AssertionError(f"prev_fmap shape {(skip.n, skip.c, skip.h, skip.w)} must match output shape {(b.n, b.c, b.h, b.w)}")
-            out = tk.groupnorm(b, *blk["n2"], groups=blk["g2"], act=self.act, skip=skip, tproj=col(tproj, blk["name"]),
-                               dtproj=col(dtproj, blk["name"]), fused=st2, prev_bias=blk["conv"].bias_name)
-            if blk["attn"] is not None:
-                out = _attention_block(tk, blk["attn"], out)
+            out = tk.groupnorm(b, *blk.n2, groups=blk.g2, act=self.act, skip=skip, tproj=col(tproj, blk.head.name),
+                               dtproj=col(dtproj, blk.head.name), fused=st2, prev_bias=blk.conv.bias_name)
+            if blk.attn is not None:
+                out = _attention_block(tk, blk.attn, self.spec.n_heads, out)
         smp = getattr(self, "_sampler", None)
         res = smp["dst"] if smp is not None else torch.empty((n, 1, 2 * out.h, 2 * out.w), dtype=torch.float32, device=dev)
         # 1 / std per member (training) or per sampler step (row of the step table selected by the device step counter)
@@ -779,8 +743,8 @@ class TrainEngine:
         t, yy, dtproj = self._time
         dscore = dscore.to(device=self.device, dtype=torch.float32).contiguous()
         da = tk.grad_like(a)
-        dwf = self._param_grad(self.final_names[0], (1, a.c, 3, 3))
-        dbf = self._param_grad(self.final_names[1], (1,))
+        dwf = self._param_grad(self.dec_layout.final_conv.weight, (1, a.c, 3, 3))
+        dbf = self._param_grad(self.dec_layout.final_conv.bias, (1,))
         dbu = self._param_grad(self.final_up.bias_name, (a.c,)) if self._final_bias_fused() else None
         ws = tk.scratch("final", _lib.query("sbgm_final_conv_backward_scratch_floats", a.c))
         call("sbgm_final_conv_backward", dscore.data_ptr(), _ptr(inv_std), a.ptr, a.plane, fmt, self.final_w.data_ptr(), da.ptr, da.plane,
@@ -801,24 +765,22 @@ class TrainEngine:
         rows = t.numel()
         # flat_order lays the nine projection weights, then the nine biases, out in head order: when they are contiguous (every
         # size is a multiple of the 64-element padding) the kernel writes the flat buffer directly, no per-head copies
-        wviews = [self._param_grad(wn, (c, self.tp.te)) for wn, _, c in self.tp_names]
-        bviews = [self._param_grad(bn, (c,)) for _, bn, c in self.tp_names]
-        in_place = all(self.offsets[self.tp_names[i + 1][0]][0] == self.offsets[self.tp_names[i][0]][0] + self.tp_names[i][2] * self.tp.te and
-                       self.offsets[self.tp_names[i + 1][1]][0] == self.offsets[self.tp_names[i][1]][0] + self.tp_names[i][2]
-                       for i in range(len(self.tp_names) - 1))
+        wviews = [self._param_grad(h.weight, tuple(self.sd[h.weight].shape)) for h in self.tp_heads]
+        bviews = [self._param_grad(h.bias, tuple(self.sd[h.bias].shape)) for h in self.tp_heads]
+        in_place = all(b.data_ptr() == a.data_ptr() + a.nbytes for views in (wviews, bviews) for a, b in zip(views, views[1:]))
         dpw = wviews[0] if in_place else torch.empty_like(pw)
         dpb = bviews[0] if in_place else torch.empty_like(pb)
-        dlab = self._param_grad(self.label_name, tuple(self.sd[self.label_name].shape)) if (self.label_name and yy is not None) else None
+        lab = self.enc_layout.label_emb
+        dlab = self._param_grad(lab, tuple(self.sd[lab].shape)) if (lab and yy is not None) else None
         ws = tk.scratch("time", _lib.query("sbgm_time_embed_backward_scratch_floats", fw.shape[0], self.tp.te, rows))
         call("sbgm_time_embed_backward", dtproj.data_ptr(), t.data_ptr(), _ptr(yy), fw.data_ptr(), fw.shape[0], self.tp.te,
              _ptr(self.tp.label_emb) if yy is not None else None, 0 if dlab is None else dlab.shape[0], pw.data_ptr(), ps.data_ptr(),
              self.tp.c_total, rows, dpw.data_ptr(), dpb.data_ptr(), _ptr(dlab), ws.data_ptr(), _stream())
         if not in_place:
-            off = 0
-            for (wn, bn, c), wv, bv in zip(self.tp_names, wviews, bviews):
-                wv.copy_(dpw[off:off + c])
-                bv.copy_(dpb[off:off + c])
-                off += c
+            sizes = [len(bv) for bv in bviews]
+            for wv, bv, dw, db in zip(wviews, bviews, dpw.split(sizes), dpb.split(sizes)):
+                wv.copy_(dw)
+                bv.copy_(db)
         if sync is not None:
             sync.progress(list(self.touched)[reported:])
             sync.finish()

@@ -409,6 +409,11 @@ int sbgm_conv2d_wgrad_simt(const void* x, size_t x_plane, const void* dy, size_t
                            int w, int cin, int cout, int kh, int kw, int stride, int pad, float* workspace, void* stream);
 /* tensor cores (tcgen05, MN-major operands straight from the NHWC tensors; cin, cout multiples of 64) */
 size_t sbgm_conv2d_wgrad_tc_workspace_floats(int fmt, int n, int h, int w, int cin, int cout, int kh, int kw, int stride, int pad);
+/* How sbgm_conv2d_wgrad_tc runs this shape (host only, launches nothing): plan[8] = {kernel (0 = per-unit, 1 = 3x3 halo slab),
+ * output channels per CTA, pixel splits, tiles per split, total tiles, tile width, tile height, images per tile}.  Tiles are
+ * numbered along the output width first, then its height, then the images; split s owns tiles [s * tiles per split, ...) and the
+ * last split may be short.  Nonzero (sbgm_last_error) for a shape sbgm_conv2d_wgrad_tc rejects. */
+int sbgm_conv2d_wgrad_tc_plan(int fmt, int n, int h, int w, int cin, int cout, int kh, int kw, int stride, int pad, int* plan);
 int sbgm_conv2d_wgrad_tc(const void* x, size_t x_plane, const void* dy, size_t dy_plane, float* dweight_oihw, int fmt,
                          int n, int h, int w, int cin, int cout, int kh, int kw, int stride, int pad, float* workspace, void* stream);
 /* sum workspace[splits][cout][taps*cin] over the splits in a fixed order into OIHW */

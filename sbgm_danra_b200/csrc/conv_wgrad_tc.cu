@@ -386,6 +386,29 @@ extern "C" size_t sbgm_conv2d_wgrad_tc_workspace_floats(int fmt, int n, int h, i
   return static_cast<size_t>(splits) * cout * p.K;
 }
 
+extern "C" int sbgm_conv2d_wgrad_tc_plan(int fmt, int n, int h, int w, int cin, int cout, int kh, int kw, int stride, int pad, int* plan) {
+  SBGM_REQUIRE(fmt == SBGM_FMT_BF16 || fmt == SBGM_FMT_BF16X2, "conv2d_wgrad_tc_plan: format %d is not a tensor-core format", fmt);
+  SBGM_REQUIRE(cin % 64 == 0 && cout % 64 == 0, "conv2d_wgrad_tc_plan: cin=%d and cout=%d must be multiples of 64", cin, cout);
+  SBGM_REQUIRE(stride >= 1 && stride <= 8, "conv2d_wgrad_tc_plan: stride %d unsupported", stride);
+  const int ho = (h + 2 * pad - kh) / stride + 1, wo = (w + 2 * pad - kw) / stride + 1;
+  SBGM_REQUIRE(ho > 0 && wo > 0, "conv2d_wgrad_tc_plan: empty output");
+  if (wgrad_slab_ok(fmt, n, h, w, cin, cout, kh, kw, stride, pad)) {
+    WgradSlabParams sp;
+    int ss = 0;
+    wgrad_slab_plan(n, h, w, cin, cout, &sp, &ss);
+    const int out[8] = {1, 64, ss, sp.tiles_per_split, sp.total_tiles, 8, 16, 1};
+    for (int i = 0; i < 8; ++i) plan[i] = out[i];
+    return 0;
+  }
+  WgradParams p;
+  int bn = 0, splits = 0;
+  wgrad_tc_plan(n, ho, wo, cin, cout, kh, kw, fmt, &p, &bn, &splits);
+  SBGM_REQUIRE(p.w_tile * stride <= 256 && p.h_tile * stride <= 256, "conv2d_wgrad_tc_plan: TMA box too large for stride %d", stride);
+  const int out[8] = {0, bn, splits, p.tiles_per_split, p.total_tiles, p.w_tile, p.h_tile, p.n_tile};
+  for (int i = 0; i < 8; ++i) plan[i] = out[i];
+  return 0;
+}
+
 extern "C" int sbgm_conv2d_wgrad_tc(const void* x, size_t x_plane, const void* dy, size_t dy_plane, float* dweight_oihw, int fmt,
                                     int n, int h, int w, int cin, int cout, int kh, int kw, int stride, int pad, float* workspace,
                                     void* stream) {

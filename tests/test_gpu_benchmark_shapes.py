@@ -5,7 +5,9 @@ The small-batch tests in test_gpu_model.py / test_gpu_train.py pick other tiles,
 
   C2  score of 64 members, 128x128, Cin = 2 (the EM ensemble's network evaluation), every tensor-core precision
   C3  128x128, Cin = 7 + season labels, predictor-corrector, bf16 (and the fp32-class modes), 8 members x 3 steps
-  C4  DSM loss + every parameter gradient at 128x128, batch 8, train-mode BatchNorm, bf16 and the fp32-class modes
+  C4  DSM loss + every parameter gradient at 128x128, train-mode BatchNorm, bf16 and the fp32-class modes, at batch 8 and at
+      bench.py's batch of 64 (where five bf16 weight gradients of the decoder take the halo-slab kernel);
+      and the bf16 step at batch 64 replayed from its CUDA graphs, bit for bit
 
 bf16 has no reference implementation to be "equal" to (the reference is fp32-only, sbgm/training.py:325-343 has its AMP branch
 commented out); its yardstick is the oracle itself run under `torch.autocast(bfloat16)`: the kernels' bf16 error must stay
@@ -140,35 +142,85 @@ def _whole(g, ref, keys):
     return rel_l2(torch.cat([g[k].reshape(-1) for k in keys]), torch.cat([ref[k].reshape(-1) for k in keys]))
 
 
-@pytest.fixture(scope="module")
-def c4_oracle():
-    """C4 shape per sample (128x128, Cin = 7 + seasons, SDF weighting, train-mode BatchNorm), batch 8: fp32 oracle loss and
-    gradients, and the same under CPU bf16 autocast (the yardstick of the bf16 mode)."""
+def _c4_oracle(batch):
+    """C4 shape per sample (128x128, Cin = 7 + seasons, SDF weighting, train-mode BatchNorm): fp32 oracle loss and gradients,
+    and the same under CPU bf16 autocast (the yardstick of the bf16 mode)."""
     from oracle.synth import config_for, synth_batch, synth_state_dict
     ck = dict(n_lr=2, geo=True, seasons=True)
     cfg = config_for(**ck)
     sd = synth_state_dict(cfg)
-    b = synth_batch(batch=8, size=128, **ck)
+    b = synth_batch(batch=batch, size=128, **ck)
     loss, grads = _oracle_dsm(cfg, sd, b, 2025, True)
     loss_ac, grads_ac = _oracle_dsm(cfg, sd, b, 2025, True, autocast=True)
     keys = sorted(grads)
     return cfg, sd, b, loss, grads, keys, abs(float(loss_ac - loss)) / abs(float(loss)), _whole(grads_ac, grads, keys)
 
 
-@pytest.mark.parametrize("precision", ["bf16x3", "bf16"])
-def test_c4_dsm_loss_and_gradient_128x128_batch8_matches_oracle(c4_oracle, precision):
-    cfg, sd, b, loss, grads, keys, ac_loss_err, ac_grad_err = c4_oracle
+@pytest.fixture(scope="module")
+def c4_oracle():
+    return _c4_oracle(8)
+
+
+@pytest.fixture(scope="module")
+def c4_oracle_batch64():
+    return _c4_oracle(64)
+
+
+def _check_c4(oracle, precision):
+    cfg, sd, b, loss, grads, keys, ac_loss_err, ac_grad_err = oracle
     got_loss, got = _ours_dsm(cfg, sd, b, 2025, precision, True)
     assert sorted(got) == keys, "the set of parameters that receive a gradient differs from the reference's"
     lerr = abs(float(got_loss - loss)) / abs(float(loss))
     gerr = _whole(got, grads, keys)
     worst = max((rel_l2(got[k], grads[k]), k) for k in keys)
-    print(f"C4 DSM 8 x 128x128 [{precision}]: loss rel {lerr:.2e}, whole-gradient rel-L2 {gerr:.3e}, worst {worst[1]} {worst[0]:.2e}; "
-          f"autocast-bf16 oracle: loss rel {ac_loss_err:.2e}, whole-gradient {ac_grad_err:.3e}")
+    print(f"C4 DSM {b.x.shape[0]} x 128x128 [{precision}]: loss rel {lerr:.2e}, whole-gradient rel-L2 {gerr:.3e}, worst {worst[1]} "
+          f"{worst[0]:.2e}; autocast-bf16 oracle: loss rel {ac_loss_err:.2e}, whole-gradient {ac_grad_err:.3e}")
     if precision == "bf16":
         assert lerr < max(2 * ac_loss_err, 1e-3) and gerr < 2 * ac_grad_err
     else:
         assert lerr < 1e-4 and gerr < 1e-3 and worst[0] < 2e-2      # worst = a 128-element BatchNorm bias (measured 8.5e-3)
+
+
+@pytest.mark.parametrize("precision", ["bf16x3", "bf16"])
+def test_c4_dsm_loss_and_gradient_128x128_batch8_matches_oracle(c4_oracle, precision):
+    _check_c4(c4_oracle, precision)
+
+
+@pytest.mark.parametrize("precision", ["bf16x3", "bf16"])
+def test_c4_dsm_loss_and_gradient_128x128_batch64_matches_oracle(c4_oracle_batch64, precision):
+    """The batch bench.py times: in bf16 the weight gradients of the conv_up of decoder blocks 1-3, of decoder block 3's conv and
+    of the final conv_up run the halo-slab kernel."""
+    _check_c4(c4_oracle_batch64, precision)
+
+
+def test_c4_graph_replay_at_batch64_is_bitwise_reproducible():
+    """The step bench.py times (bf16, train mode, batch 64): steps 1-2 run the eager engine, steps 3-5 replay the captured forward
+    and backward CUDA graphs.  Same inputs, same Philox seed, no optimizer step -> the loss and every gradient equal step 1's bit
+    for bit.  In train mode BatchNorm normalises with batch statistics, so the running buffers that move between steps do not
+    enter the gradients."""
+    from oracle.synth import config_for, synth_batch, synth_state_dict
+    from sbgm_danra_b200 import score_sampling
+    from sbgm_danra_b200._smoke import build_model
+    from sbgm_danra_b200.score_unet import loss_fn, marginal_prob_std_fn
+    ck = dict(n_lr=2, geo=True, seasons=True)
+    cfg = config_for(**ck)
+    net = build_model(cfg, synth_state_dict(cfg), "bf16", DEV).train()
+    b = synth_batch(batch=64, size=128, **ck)
+    snaps = []
+    for step in range(5):
+        score_sampling.manual_seed(3)
+        net.zero_grad(set_to_none=True)
+        loss = loss_fn(net, _cuda(b.x), marginal_prob_std_fn, y=_cuda(b.y), cond_img=_cuda(b.cond_img), lsm_cond=_cuda(b.lsm_cond),
+                       topo_cond=_cuda(b.topo_cond), sdf_cond=_cuda(b.sdf_cond))
+        loss.backward()
+        snaps.append((loss.item(), {k: p.grad.clone() for k, p in net.named_parameters() if p.grad is not None}))
+    runner = next(iter(net._train_runners.values()))
+    assert runner.g_fwd is not None and runner.g_bwd is not None, "the step was never captured"
+    for loss_k, grads_k in snaps[1:]:
+        assert loss_k == snaps[0][0]
+        assert grads_k.keys() == snaps[0][1].keys()
+        for k in grads_k:
+            assert torch.equal(grads_k[k], snaps[0][1][k]), k
 
 
 @pytest.mark.parametrize("mode", ["train", "eval"])

@@ -234,38 +234,14 @@ def test_conv_backward(E, T, prec, case):
     tk.tape.add(ya, act_of(E, dy, fmt))
     run_tape(tk)
     e_dx = rel_l2(tk.tape.grads[xa.buf.data_ptr()].to_nchw().cpu(), x.grad)
-    e_dw = rel_l2(grads["w"].cpu(), wr.grad)
+    # dW is fp32 sums of exact products of the stored x and dy (bf16x3 drops lo x lo, ~2^-16): gated against float64, not
+    # at ftol.  dx is rounded to the activation format on output, so it keeps the forward's gate.
+    dw_ref = torch.nn.grad.conv2d_weight(x.detach().double(), wt.shape, dy.double(), stride=stride, padding=pad)
+    e_dw = rel_l2(grads["w"].cpu(), dw_ref)
     print(f"{case} [{prec}] dx {e_dx:.2e} dW {e_dw:.2e}")
-    assert e_dx < ftol and e_dw < ftol
+    assert e_dx < ftol and e_dw < {"fp32": 1e-5, "bf16x3": 5e-5, "bf16": 1e-5}[prec]
     if bias:
         assert rel_l2(grads["b"].cpu(), br.grad) < ftol
-
-
-@pytest.mark.parametrize("prec", ["bf16x3", "bf16"])
-@pytest.mark.parametrize("geom", [(4, 32, 32, 64, 64, 3, 1, 1),
-                                  # bf16: the halo-slab kernel (3x3 / stride 1, maps tileable by 16 rows x 8 columns) -- two channel
-                                  # blocks, two output blocks, one tile per image, an odd image count over several pixel splits
-                                  (3, 16, 8, 128, 128, 3, 1, 1), (5, 48, 24, 64, 192, 3, 1, 1), (2, 32, 32, 256, 64, 3, 1, 1),
-                                  (2, 24, 16, 64, 64, 3, 1, 1),          # 24 rows: not slab-tileable, the per-unit kernel
-                                  (2, 16, 16, 64, 128, 3, 2, 1)])        # strided: the per-unit kernel
-def test_wgrad_tc_matches_simt(E, prec, geom):
-    """The tensor-core weight gradient against the CUDA-core one on identical stored operands."""
-    from sbgm_danra_b200 import _lib
-    from sbgm_danra_b200._lib import call
-    fmt = FMTS[prec]
-    n, h, w, cin, cout, k, stride, pad = geom
-    ho, wo = (h + 2 * pad - k) // stride + 1, (w + 2 * pad - k) // stride + 1
-    xa, da = act_of(E, gen(n, cin, h, w, seed=1), fmt), act_of(E, gen(n, cout, ho, wo, seed=2), fmt)
-    st = torch.cuda.current_stream().cuda_stream
-    out = []
-    for name in ("tc", "simt"):
-        args = (n, h, w, cin, cout, k, k, stride, pad)
-        nws = _lib.query(f"sbgm_conv2d_wgrad_{name}_workspace_floats", *(((fmt,) + args) if name == "tc" else args))
-        ws = torch.empty(nws, device=DEV)
-        dw = torch.zeros(cout, cin, k, k, device=DEV)
-        call(f"sbgm_conv2d_wgrad_{name}", xa.ptr, xa.plane, da.ptr, da.plane, dw.data_ptr(), fmt, *args, ws.data_ptr(), st)
-        out.append(dw.cpu())
-    assert rel_l2(out[0], out[1]) < (5e-5 if prec == "bf16x3" else 1e-5)
 
 
 @pytest.mark.parametrize("prec", ["fp32", "bf16x3"])

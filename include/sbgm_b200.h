@@ -422,6 +422,17 @@ int sbgm_wgrad_reduce(const float* workspace, int splits, int cout, int taps, in
 size_t sbgm_stem_wgrad_workspace_floats(int cin);
 int sbgm_stem_wgrad(const float* x, const float* planes, int np, int cc, const void* df, size_t df_plane, int fmt, float* dweight_oihw,
                     int n, int h, int w, float* workspace, void* stream);
+/* Encoder.conv1 data gradient from df [n,h/2,w/2,64] (fmt): dx [n,1,h,w] and dplanes [np,cc,h,w], fp32 NCHW, each nullable;
+ * np == 1 (planes shared by the batch): dplanes is the sum over the batch, built in `workspace` (the size below, 0 otherwise).
+ * cc <= 15.  CUDA cores, any format, weight = conv1.weight as fp32 OIHW [64][cc+1][8][8]: */
+size_t sbgm_stem_dgrad_workspace_floats(int np, int cc, int n, int h, int w);
+int sbgm_stem_dgrad_simt(const void* df, size_t df_plane, int fmt, const float* w_oihw, float* dx, float* dplanes, int np, int cc, int n,
+                         int h, int w, float* workspace, void* stream);
+/* tensor cores (tcgen05), bf16 and split bf16: w_packed [4 parity classes (py * 2 + px)][planes][16][16 taps * 64] bf16, planes
+ * w_plane elements apart, class c = sbgm_pack_weight(conv1.weight zero-padded to 16 input channels, transpose = 1, taps r * 8 + s
+ * for r = 7 - py - 2 ky, s = 7 - px - 2 kx, ky and kx = 0..3 in that order) */
+int sbgm_stem_dgrad_tc(const void* df, size_t df_plane, int fmt, const void* w_packed, size_t w_plane, float* dx, float* dplanes,
+                       int np, int cc, int n, int h, int w, float* workspace, void* stream);
 /* Decoder.final_layer.conv (cin -> 1, 3x3) + the 1/std scaling, backward: g = dscore * inv_std[n];
  * da [n,h,w,cin] (fmt), dweight_oihw[1][cin][3][3], dbias[1]; weight_tap_ci = fp32 [9][cin].  dbias_up[cin] (nullable) = da
  * summed over n,h,w: the bias gradient of the convolution that produced `a` (final_layer.conv_up), free in the same pass

@@ -35,6 +35,9 @@ inline cudaStream_t as_stream(void* s) { return reinterpret_cast<cudaStream_t>(s
 void note_launch_error(cudaError_t e);
 bool pdl_enabled();
 int resident_blocks(const void* kern, int block, size_t smem);   // blocks of `kern` resident at once on the GPU (elementwise.cu)
+// out[i] = sum over b < n of per_sample[b * per + i] in batch order (conv_grad_simt.cu; the stem data gradient of planes shared by
+// the batch)
+int stem_dgrad_batch_sum(const float* per_sample, float* out, int n, size_t per, cudaStream_t st);
 #ifdef __CUDACC__
 __device__ __forceinline__ void pdl_grid_sync() {
   // wait only: the dependents are released when this grid's blocks exit (implicit trigger).  Releasing them at the top

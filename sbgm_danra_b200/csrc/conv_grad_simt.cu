@@ -215,6 +215,61 @@ __global__ void stem_wgrad_reduce_kernel(const float* __restrict__ ws, int cin, 
   }
 }
 
+// ---- stem dgrad: d(x || planes)[b][ci][iy][ix] = sum_{r,s,co} df[b][oy][ox][co] * w[co][ci][r][s],  2 oy + r - 3 = iy ------------
+// Thread = one input pixel of one parity class (blockIdx.y): its 16 taps are r = 7 - py - 2 ky at df row jy + py - 2 + ky (same
+// for the columns), so a warp's weight loads are uniform.  The fp32 path, and the cross-check of stem_dgrad_tc.cu.
+template <int FMT>
+__global__ void __launch_bounds__(128)
+stem_dgrad_simt_kernel(const void* __restrict__ df, size_t df_plane, const float* __restrict__ w_oihw, float* __restrict__ dx,
+                       float* __restrict__ dpl, int n, int cc, int h, int w) {
+  pdl_grid_sync();
+  const int hh = h / 2, wh = w / 2, cin = cc + 1;
+  const int py = blockIdx.y >> 1, px = blockIdx.y & 1;
+  const size_t total = static_cast<size_t>(n) * hh * wh;
+  for (size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; i < total; i += static_cast<size_t>(gridDim.x) * blockDim.x) {
+    const int jx = static_cast<int>(i % wh), jy = static_cast<int>((i / wh) % hh), b = static_cast<int>(i / (static_cast<size_t>(wh) * hh));
+    float acc[16];
+#pragma unroll
+    for (int c = 0; c < 16; ++c) acc[c] = 0.0f;
+    for (int ky = 0; ky < 4; ++ky) {
+      const int oy = jy + py - 2 + ky, r = 7 - py - 2 * ky;
+      if (oy < 0 || oy >= hh) continue;
+      for (int kx = 0; kx < 4; ++kx) {
+        const int ox = jx + px - 2 + kx, s = 7 - px - 2 * kx;
+        if (ox < 0 || ox >= wh) continue;
+        const size_t base = ((static_cast<size_t>(b) * hh + oy) * wh + ox) * 64;
+        const float* wt = w_oihw + r * 8 + s;
+        for (int v8 = 0; v8 < 8; ++v8) {
+          float g[8];
+          Act<FMT>::load8(df, df_plane, base + v8 * 8, g);
+#pragma unroll
+          for (int e = 0; e < 8; ++e) {
+            const float* wc = wt + static_cast<size_t>(v8 * 8 + e) * cin * 64;
+#pragma unroll
+            for (int c = 0; c < 16; ++c)
+              if (c < cin) acc[c] = fmaf(g[e], __ldg(wc + c * 64), acc[c]);
+          }
+        }
+      }
+    }
+    const size_t hw = static_cast<size_t>(h) * w, pix = static_cast<size_t>(2 * jy + py) * w + 2 * jx + px;
+    if (dx) dx[b * hw + pix] = acc[0];
+    if (dpl) {
+#pragma unroll
+      for (int c = 1; c < 16; ++c)
+        if (c < cin) dpl[(static_cast<size_t>(b) * cc + c - 1) * hw + pix] = acc[c];
+    }
+  }
+}
+__global__ void batch_sum_kernel(const float* __restrict__ src, float* __restrict__ out, int n, size_t per) {
+  pdl_grid_sync();
+  for (size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; i < per; i += static_cast<size_t>(gridDim.x) * blockDim.x) {
+    float acc = 0.0f;
+    for (int b = 0; b < n; ++b) acc += src[b * per + i];
+    out[i] = acc;
+  }
+}
+
 // ---- final convolution (cin -> 1, 3x3, pad 1) backward, fused with the 1/std scaling ---------------------
 // g[n,y,x] = dscore[n,y,x] * inv_std[n]
 template <int FMT>
@@ -490,6 +545,11 @@ static void wgrad_simt_plan(int n, int ho, int wo, int cin, int cout, int taps, 
   *per = static_cast<int>(pp);
 }
 
+int stem_dgrad_batch_sum(const float* per_sample, float* out, int n, size_t per, cudaStream_t st) {
+  launch_k((batch_sum_kernel), cgrid_for(per, 256), 256, 0, st, per_sample, out, n, per);
+  return check_launch("stem_dgrad_batch_sum");
+}
+
 }  // namespace sbgm
 
 using namespace sbgm;
@@ -549,6 +609,28 @@ int sbgm_stem_wgrad(const float* x, const float* planes, int np, int cc, const v
   SBGM_DISPATCH_FMT(fmt, (launch_k((stem_wgrad_kernel<FMT>), grid, 256, 0, st, x, planes, np, cc, df, df_plane, workspace, n, h, w)));
   launch_k((stem_wgrad_reduce_kernel), cgrid_for(static_cast<size_t>(cin) * 4096, 256), 256, 0, st, workspace, cin, dweight_oihw);
   return check_launch("stem_wgrad");
+}
+
+size_t sbgm_stem_dgrad_workspace_floats(int np, int cc, int n, int h, int w) {
+  return np == 1 && n > 1 ? static_cast<size_t>(n) * cc * h * w : 0;
+}
+
+int sbgm_stem_dgrad_simt(const void* df, size_t df_plane, int fmt, const float* w_oihw, float* dx, float* dplanes, int np, int cc, int n,
+                         int h, int w, float* workspace, void* stream) {
+  SBGM_REQUIRE(h % 2 == 0 && w % 2 == 0 && h > 0 && w > 0, "stem_dgrad_simt: h=%d and w=%d must be even", h, w);
+  SBGM_REQUIRE(cc >= 0 && cc < 16, "stem_dgrad_simt: %d conditioning channels (at most 15)", cc);
+  SBGM_REQUIRE(np == 1 || np == n, "stem_dgrad_simt: planes batch %d must be 1 or %d", np, n);
+  SBGM_REQUIRE(dplanes == nullptr || (cc > 0 && (np == n || n == 1 || workspace != nullptr)),
+               "stem_dgrad_simt: dplanes needs cc > 0 and, for planes shared by the batch, a workspace");
+  cudaStream_t st = as_stream(stream);
+  const bool sum_batch = dplanes != nullptr && np == 1 && n > 1;
+  float* dpl = sum_batch ? workspace : dplanes;
+  const size_t total = static_cast<size_t>(n) * (h / 2) * (w / 2);
+  dim3 grid(cgrid_for(total, 128, 148 * 8), 4);
+  SBGM_DISPATCH_FMT(fmt, (launch_k((stem_dgrad_simt_kernel<FMT>), grid, 128, 0, st, df, df_plane, w_oihw, dx, dpl, n, cc, h, w)));
+  const int rc = check_launch("stem_dgrad_simt");
+  if (rc != 0 || !sum_batch) return rc;
+  return stem_dgrad_batch_sum(workspace, dplanes, n, static_cast<size_t>(cc) * h * w, st);
 }
 
 static bool final_fused_ok(int cin) {       // 8, 16 or 32 channel vectors: 32, 16 or 8 pixel lanes, a g tile of <= 512 values

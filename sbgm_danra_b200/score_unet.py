@@ -474,7 +474,9 @@ class ScoreNet(nn.Module):
         needs_grad = False
         if torch.is_grad_enabled() or self.training:
             names, params, _, bn_modules = self._member_lists()
-            needs_grad = torch.is_grad_enabled() and any(p.requires_grad for p in params)
+            # the differentiable path also when only inputs want a gradient (a frozen model under torch.autograd.grad)
+            needs_grad = torch.is_grad_enabled() and (any(p.requires_grad for p in params) or any(
+                v is not None and v.requires_grad for v in (x, cond_img, lsm_cond, topo_cond)))
         if needs_grad or self.training:
             # training graph: unfolded BatchNorm (batch statistics when .training), backward tape (train_engine.py)
             with torch.cuda.device(dev):
@@ -484,7 +486,7 @@ class ScoreNet(nn.Module):
                 std = self.marginal_prob_std(t)
                 pre = bool(getattr(self, "debug_pre_sigma_div", True))
                 inv_std = None if pre else (1.0 / std.float()).contiguous()
-                out = _ScoreNetFn.apply(self, x, t, y, planes, inv_std, names, *params)
+                out = _ScoreNetFn.apply(self, x, t, y, planes, inv_std, names, torch.is_grad_enabled(), *params)
                 if self.training:
                     torch._foreach_add_([m.num_batches_tracked for m in bn_modules], 1)
                 if pre:
@@ -526,14 +528,18 @@ class _ScoreNetFn(torch.autograd.Function):
     (train_engine.TrainEngine); replaces torch autograd over sbgm/score_unet.py:829-879."""
 
     @staticmethod
-    def forward(ctx, model, x, t, y, planes, inv_std, names, *params):
+    def forward(ctx, model, x, t, y, planes, inv_std, names, grad_mode, *params):
         from .train_engine import TrainEngine, TrainRunner
         buffers = model._member_lists()[2]
         sync = getattr(model, "_grad_sync", None)
         # the captured graphs bake in the gradient exchange: a runner belongs to one GradSync object (parallel.attach / detach)
         sync_key = None if sync is None else (id(sync), bool(sync.sync_bn), sync.world)
+        # which gradients backward produces: (x, planes) and whether the parameters' (all of them as soon as one wants one)
+        input_grads = (grad_mode and ctx.needs_input_grad[1], grad_mode and ctx.needs_input_grad[4])
+        param_grads = any(ctx.needs_input_grad[8:]) or not any(input_grads)
         key = (model.precision, model.training, tuple(x.shape), None if planes is None else tuple(planes.shape), y is None,
-               inv_std is None, str(x.device), tuple(p.data_ptr() for p in params), tuple(b.data_ptr() for _, b in buffers), sync_key)
+               inv_std is None, str(x.device), tuple(p.data_ptr() for p in params), tuple(b.data_ptr() for _, b in buffers), sync_key,
+               input_grads, param_grads)
         runners = model.__dict__.setdefault("_train_runners", {})
         runner = runners.get(key)
         if runner is None:
@@ -545,7 +551,7 @@ class _ScoreNetFn(torch.autograd.Function):
             def make_engine():
                 tensors = dict(zip(names, params))
                 tensors.update(buffers)
-                return TrainEngine(tensors, spec, precision, device, bn_train=training)
+                return TrainEngine(tensors, spec, precision, device, bn_train=training, input_grads=input_grads, param_grads=param_grads)
             runners.clear()                       # one live configuration at a time (the graphs pin GBs of activations)
             runner = runners[key] = TrainRunner(make_engine, use_graphs=os.environ.get("SBGM_B200_TRAIN_GRAPHS", "1") != "0")
         if runner.eng is not None:                # captured step: its forward graph re-zeroes the flat gradient buffer
@@ -574,7 +580,8 @@ class _ScoreNetFn(torch.autograd.Function):
         for n in names:
             g = grads.get(n)
             out.append(None if g is None else (g.view(g.shape) if views else g))
-        return (None,) * 7 + tuple(out)
+        from .train_engine import DPLANES, DX
+        return (None, grads.get(DX), None, None, grads.get(DPLANES), None, None, None) + tuple(out)
 
 
 class _DSMLossFn(torch.autograd.Function):

@@ -26,6 +26,8 @@ from .engine import (ACTS, BN_EPS, GN_EPS, LN_EPS, PRECISIONS, Act, Affine, Attn
                      pack_transpose, stem_matrix)
 
 BN_MOMENTUM = 0.1
+# keys of the input gradients in the dict TrainEngine.backward returns (next to the parameter names)
+DX, DPLANES = "input:x", "input:planes"
 # "fp16x2" is an inference storage format (engine.py); a model set to it trains on the bf16x3 kernels
 TRAIN_PRECISIONS = dict(PRECISIONS, fp16x2=FMT_BF16X2)
 
@@ -65,12 +67,14 @@ class PackPlan:
         self.fmt = fmt
         self.jobs: List[Tuple[torch.Tensor, torch.Tensor, int, int, int, List[int], bool]] = []
 
-    def add(self, w4: torch.Tensor, taps: Sequence[int], transpose: bool) -> torch.Tensor:
+    def add(self, w4: torch.Tensor, taps: Sequence[int], transpose: bool, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """`out`: [planes][o][taps * i] bf16 destination (a slice of a larger table), else a new tensor."""
         cout, cin, kh, kw = w4.shape
         w4 = w4.contiguous()
         oo, ii = (cin, cout) if transpose else (cout, cin)
         planes = 2 if self.fmt == FMT_BF16X2 else 1
-        out = torch.empty((planes, oo, len(taps) * ii), dtype=torch.bfloat16, device=w4.device)
+        if out is None:
+            out = torch.empty((planes, oo, len(taps) * ii), dtype=torch.bfloat16, device=w4.device)
         self.jobs.append((w4, out, cout, cin, kh * kw, list(taps), transpose))
         return out if planes == 2 else out[0]
 
@@ -84,7 +88,7 @@ class PackPlan:
             table = (_PackJob * len(small))()
             for k, (w4, out, cout, cin, khw, taps, tr) in enumerate(small):
                 e = table[k]
-                e.w, e.out, e.out_plane = w4.data_ptr(), out.data_ptr(), out[0].numel()
+                e.w, e.out, e.out_plane = w4.data_ptr(), out.data_ptr(), out.stride(0)
                 e.cout, e.cin, e.khw, e.ntaps, e.transpose = cout, cin, khw, len(taps), int(tr)
                 for t, v in enumerate(taps):
                     e.taps[t] = v
@@ -97,6 +101,23 @@ def _dgrad_taps(k: int, stride: int, pad: int, par: int):
     offset d into dy: input index i = stride * j + par receives dy[j + d] * w[r] with r = par + pad - stride * d."""
     ds = sorted(d for d in range(-k, k + 1) if 0 <= par + pad - stride * d < k)
     return ds, [par + pad - stride * d for d in ds]
+
+
+def stem_dgrad_taps(py: int, px: int) -> List[int]:
+    """Flat taps r * 8 + s of Encoder.conv1 (8x8, stride 2, pad 3) that reach input pixels of parity (py, px), in the order of
+    sbgm_stem_dgrad_tc's K blocks (increasing offset into df)."""
+    return [r * 8 + s for r in _dgrad_taps(8, 2, 3, py)[1] for s in _dgrad_taps(8, 2, 3, px)[1]]
+
+
+def stem_dgrad_weight(plan: PackPlan, w1: torch.Tensor) -> torch.Tensor:
+    """sbgm_stem_dgrad_tc's weight table [4 classes][planes][16][16 * 64]: per parity class (py * 2 + px) conv1.weight, zero-padded
+    to 16 input channels, transposed over the class's taps.  Registered on `plan` (filled by plan.run())."""
+    w16 = torch.zeros((64, 16, 8, 8), dtype=torch.float32, device=w1.device)
+    w16[:, :w1.shape[1]] = w1
+    table = torch.empty((4, 2 if plan.fmt == FMT_BF16X2 else 1, 16, 16 * 64), dtype=torch.bfloat16, device=w1.device)
+    for cls in range(4):
+        plan.add(w16, stem_dgrad_taps(cls >> 1, cls & 1), True, out=table[cls])
+    return table
 
 
 class ConvLayer:
@@ -196,9 +217,11 @@ class Tape:
 class TrainKernels:
     """Forward ops that record their backward on a tape."""
 
-    def __init__(self, fmt: int, device, flat_grad: Callable[[str, Tuple[int, ...]], torch.Tensor]) -> None:
-        """`flat_grad(name, shape)`: the gradient view of a parameter, reported as produced at once."""
-        self.fmt, self.device = fmt, device
+    def __init__(self, fmt: int, device, flat_grad: Callable[[str, Tuple[int, ...]], torch.Tensor], params: bool = True) -> None:
+        """`flat_grad(name, shape)`: the gradient view of a parameter, reported as produced at once.  `params=False`: only data
+        gradients are wanted -- launches whose only product is a parameter gradient are skipped, and `flat_grad` hands out
+        scratch for the parameter gradients that kernels produce next to a data gradient."""
+        self.fmt, self.device, self.params = fmt, device, params
         self.k = Kernels(fmt, device)
         self.tape: Optional[Tape] = None
         self.param_grad = flat_grad
@@ -269,7 +292,7 @@ class TrainKernels:
             self._conv_backward(x, dy, layer, stride, pad, need_dx, bias_grad)
             if residual is not None:
                 tape.add(residual, dy)
-            if dtproj is not None:
+            if dtproj is not None and self.params:
                 self.channel_sums(dy, dtproj=dtproj)
 
         tape.record(backward, x, y)
@@ -281,9 +304,11 @@ class TrainKernels:
         fmt, st = self.fmt, _stream()
         n, h, w = x.n, x.h, x.w
         cin, cout, kh, kw = layer.cin, layer.cout, layer.kh, layer.kw
-        if layer.bias_name is not None and bias_grad:
-            self.channel_sums(dy, dbias=self.param_grad(layer.bias_name, (cout,)))
-        tc = self.wgrad(x, dy, self.param_grad(layer.name, layer.shape), cin, cout, kh, kw, stride, pad)
+        if self.params:
+            if layer.bias_name is not None and bias_grad:
+                self.channel_sums(dy, dbias=self.param_grad(layer.bias_name, (cout,)))
+            self.wgrad(x, dy, self.param_grad(layer.name, layer.shape), cin, cout, kh, kw, stride, pad)
+        tc = fmt != FMT_F32 and cin % 64 == 0 and cout % 64 == 0          # the data gradient takes the weight gradient's route
         if not need_dx:
             return
         tape = self.tape
@@ -458,9 +483,10 @@ class TrainKernels:
             dy = tape.pop(y)
             if dy is None:
                 return
-            self.channel_sums(dy, dbias=self.param_grad(layer.bias_name, (layer.cout,)))
-            # C: input dy-grid (cout channels), output x-grid
-            self.wgrad(dy, x, self.param_grad(layer.name, layer.shape), layer.cout, layer.cin, 2, 2, 2, 0)
+            if self.params:
+                self.channel_sums(dy, dbias=self.param_grad(layer.bias_name, (layer.cout,)))
+                # C: input dy-grid (cout channels), output x-grid
+                self.wgrad(dy, x, self.param_grad(layer.name, layer.shape), layer.cout, layer.cin, 2, 2, 2, 0)
             tape.add(x, self.k.conv(dy, layer.back, stride=2, pad=0))
 
         tape.record(backward, x, y)
@@ -527,11 +553,15 @@ class TrainEngine:
     statistics are updated in place when `bn_train` is set."""
 
     def __init__(self, params: Dict[str, torch.Tensor], spec: UNetSpec, precision: str, device, bn_train: bool,
-                 encoder_only: bool = False) -> None:
+                 encoder_only: bool = False, input_grads: Tuple[bool, bool] = (False, False), param_grads: bool = True) -> None:
         """`encoder_only`: `params` is the standalone Encoder's own state dict and `forward` returns its five feature maps
-        (`Encoder.forward` in .train(): batch statistics, running statistics updated; nothing is differentiated)."""
+        (`Encoder.forward` in .train(): batch statistics, running statistics updated; nothing is differentiated).
+        `input_grads` = (x, planes): backward also returns the gradient of x / of the conditioning planes (keys DX, DPLANES).
+        `param_grads=False`: backward computes data gradients only -- no flat gradient buffer, no weight-gradient launches, no
+        gradient exchange."""
         device = engine_device(precision, device)
         self.spec, self.device, self.fmt, self.bn_train = spec, device, TRAIN_PRECISIONS[precision], bn_train
+        self.input_grads, self.param_grads = tuple(bool(v) for v in input_grads), param_grads
         self.encoder_only = encoder_only
         self.enc_layout = encoder_layout(spec, "") if encoder_only else encoder_layout(spec)
         self.dec_layout = None if encoder_only else decoder_layout(spec)
@@ -550,13 +580,19 @@ class TrainEngine:
         self.flat_numel = off
         self.flat: Optional[torch.Tensor] = None
         self.touched: Dict[str, torch.Tensor] = {}
-        self.tk = TrainKernels(self.fmt, device, self._param_grad)
+        self._sink: Dict[str, torch.Tensor] = {}     # parameter-gradient by-products when param_grads is off
+        self.tk = TrainKernels(self.fmt, device, self._param_grad, params=param_grads)
         self.grad_sync = None      # parallel.GradSync or None
         with torch.cuda.device(device), torch.no_grad():
             self._pack()
 
     # -- parameters -------------------------------------------------------------------------------
     def _param_grad(self, name: str, shape: Tuple[int, ...]) -> torch.Tensor:
+        if not self.param_grads:
+            g = self._sink.get(name)
+            if g is None:
+                g = self._sink[name] = torch.empty(shape, dtype=torch.float32, device=self.device)
+            return g
         off, numel = self.offsets[name]
         g = self.flat[off:off + numel].view(shape)
         self.touched[name] = g
@@ -588,6 +624,8 @@ class TrainEngine:
         if fmt != FMT_F32:   # tensor-core stem: 1x1 convolution over the im2col tensor; [co][ci*64 + tap] IS conv1.weight's OIHW order
             self.stem_layer = ConvLayer(enc.stem, w1.reshape(64, self.cin * 64, 1, 1), None, fmt, plan=self.plan, need_dx=False)
             self.stem_layer.shape = tuple(w1.shape)
+        if any(self.input_grads) and fmt != FMT_F32:
+            self.stem_dgrad_w = stem_dgrad_weight(self.plan, w1)
         self.conv2, self.bn1 = self._conv_bn(enc.conv2, 2, 3)
         self.layers = [[s._replace(down=None if s.down is None else self._conv_bn(s.down, s.stride, 0), c1=self._conv_bn(s.c1, s.stride, 1),
                                    c2=self._conv_bn(s.c2, 1, 1)) for s in stage] for stage in enc.stages]
@@ -632,7 +670,7 @@ class TrainEngine:
             tproj = sampler["tproj"]
             dtproj = tproj                     # never written: no backward runs on a sampler step
         else:
-            self.flat = torch.zeros(self.flat_numel, dtype=torch.float32, device=dev)
+            self.flat = torch.zeros(self.flat_numel, dtype=torch.float32, device=dev) if self.param_grads else None
             t = t.reshape(-1).to(device=dev, dtype=torch.float32).contiguous()
             tproj = self.tp(t, yy)
             dtproj = torch.zeros_like(tproj)
@@ -642,9 +680,13 @@ class TrainEngine:
         self._time = (t, yy, dtproj)
         # Encoder.conv1 + time projection 0 (score_unet.py:310-314)
         t0 = col(tproj, "enc0")
+        self._input_grads = {}
         if fmt != FMT_F32:
             xcol = tk.k.stem_im2col(x, planes, 0, self.cin, cc)
             f1 = tk.conv(xcol, self.stem_layer, need_dx=False, tproj=t0, dtproj=col(dtproj, "enc0"))
+            if any(self.input_grads):
+                # recorded after the stem's own step, so it runs first in backward and reads df before that step consumes it
+                tape.record(lambda: self._stem_dgrad(tape.grads.get(f1.buf.data_ptr()), x, planes))
             return self._forward_rest(f1, tproj, dtproj, inv_std, n)
         f1 = Act(fmt, n, h // 2, w // 2, 64, dev)
         call("sbgm_stem_conv", x.data_ptr(), _ptr(planes), 1 if planes is None else planes.shape[0], cc, 0, self.cin,
@@ -654,6 +696,9 @@ class TrainEngine:
             df = tape.pop(f1)
             if df is None:
                 return
+            self._stem_dgrad(df, x, planes)
+            if not self.param_grads:
+                return
             tk.channel_sums(df, dtproj=col(dtproj, "enc0"))
             dw = self._param_grad(self.enc_layout.stem, (64, self.cin, 8, 8))
             ws2 = tk.scratch("stem", _lib.query("sbgm_stem_wgrad_workspace_floats", self.cin))
@@ -662,6 +707,35 @@ class TrainEngine:
 
         tape.record(stem_backward, f1)
         return self._forward_rest(f1, tproj, dtproj, inv_std, n)
+
+    def _stem_dgrad(self, df: Optional[Act], x: torch.Tensor, planes: Optional[torch.Tensor]) -> None:
+        """Encoder.conv1's data gradient: the requested ones of dx [n, 1, h, w] and dplanes [np, cc, h, w] (fp32) into
+        self._input_grads (zeros when nothing reached the stem)."""
+        want_x, want_planes = self.input_grads
+        want_planes = want_planes and planes is not None
+        if not (want_x or want_planes):
+            return
+        dx = torch.empty_like(x) if want_x else None
+        dpl = torch.empty_like(planes) if want_planes else None
+        if df is None:
+            for g in (dx, dpl):
+                if g is not None:
+                    g.zero_()
+        else:
+            n, _, h, w = x.shape
+            np_, cc = (1, 0) if planes is None else (planes.shape[0], planes.shape[1])
+            ws = self.tk.scratch("stem_dgrad", _lib.query("sbgm_stem_dgrad_workspace_floats", np_, cc, n, h, w))
+            if self.fmt == FMT_F32:
+                call("sbgm_stem_dgrad_simt", df.ptr, df.plane, self.fmt, self.sd[self.enc_layout.stem].data_ptr(), _ptr(dx), _ptr(dpl),
+                     np_, cc, n, h, w, ws.data_ptr(), _stream())
+            else:
+                wt = self.stem_dgrad_w
+                call("sbgm_stem_dgrad_tc", df.ptr, df.plane, self.fmt, wt.data_ptr(), wt.stride(1), _ptr(dx), _ptr(dpl), np_, cc, n, h, w,
+                     ws.data_ptr(), _stream())
+        if dx is not None:
+            self._input_grads[DX] = dx
+        if dpl is not None:
+            self._input_grads[DPLANES] = dpl
 
     def _forward_rest(self, f1: Act, tproj: torch.Tensor, dtproj: torch.Tensor, inv_std: Optional[torch.Tensor], n: int) -> torch.Tensor:
         tk, fmt, dev, tape = self.tk, self.fmt, self.device, self.tape
@@ -741,6 +815,7 @@ class TrainEngine:
         tk, tape, fmt = self.tk, self.tape, self.fmt
         a, inv_std = self._final
         t, yy, dtproj = self._time
+        params = self.param_grads
         dscore = dscore.to(device=self.device, dtype=torch.float32).contiguous()
         da = tk.grad_like(a)
         dwf = self._param_grad(self.dec_layout.final_conv.weight, (1, a.c, 3, 3))
@@ -750,7 +825,7 @@ class TrainEngine:
         call("sbgm_final_conv_backward", dscore.data_ptr(), _ptr(inv_std), a.ptr, a.plane, fmt, self.final_w.data_ptr(), da.ptr, da.plane,
              dwf.data_ptr(), dbf.data_ptr(), _ptr(dbu), a.n, a.h, a.w, a.c, ws.data_ptr(), _stream())
         tape.add(a, da)
-        sync = self.grad_sync
+        sync = self.grad_sync if params else None
         if sync is not None:
             sync.begin(self.flat, [(k, *self.offsets[k]) for k in self.grad_names])
         reported = 0
@@ -760,6 +835,11 @@ class TrainEngine:
                 new = list(self.touched)[reported:]
                 reported = len(self.touched)
                 sync.progress(new)
+        if not params:
+            grads = dict(self._input_grads)
+            self.tape = tk.tape = None
+            self._final = self._time = None
+            return grads
         # time embedding: one launch set for all nine projections (+ label embedding)
         fw, pw, pb, ps = self.tp._packed
         rows = t.numel()
@@ -784,7 +864,7 @@ class TrainEngine:
         if sync is not None:
             sync.progress(list(self.touched)[reported:])
             sync.finish()
-        grads = dict(self.touched)
+        grads = dict(self.touched, **self._input_grads)
         self.tape = None
         tk.tape = None
         self._final = self._time = None
@@ -958,4 +1038,5 @@ class TrainRunner:
             self.static["dout"].copy_(dout)
         self.g_bwd.replay()
         obj.release()
-        return self.grads
+        # the input gradients live in the graph's memory pool and the next replay rewrites them: hand out copies
+        return {k: (v.clone() if k in (DX, DPLANES) else v) for k, v in self.grads.items()}
